@@ -8,6 +8,8 @@ synthetic 144-byte flow records that is already resident in HBM.  Workloads (BAS
   zipf1m     configs[1]: 1 M Zipf-1.1 5-tuples
 One JSON line on stdout (rank 0).  After the timed loop the engine's output is checked against the CPU oracle on a
 fresh prefix of the same stream (`parity_checked` = flows compared bit for bit; --no-verify skips it).
+--dump-outputs DIR writes what the timed steps computed (see dump_outputs()); the inputs depend on the arguments only,
+so two builds run with the same arguments can be compared output for output.
 --impl reference times the CPU restatement of pkg/flow.Accounter (the Go reference cannot be built in this image) on
 a bounded sample of the same workload; that arm never loads the product library.
 """
@@ -217,6 +219,23 @@ def record_order(r):
     return np.lexsort((h2, h1))
 
 
+DUMP_FLOWS = 1 << 15           # --dump-outputs: 32768 flows x 144 bytes as float32 = 18.9 MB (+ 32 MB of count-min)
+
+
+def dump_outputs(out_dir, recs, sketch=None):
+    """--dump-outputs: the flow table the timed steps left, as a caller of fa_evict receives it ((n,144) records; float32
+    holds every byte exactly).  A larger table is sampled by key hash: the DUMP_FLOWS flows that come first in
+    record_order(), so the sample depends on the flows alone, not on the slots the table keeps them in.  With the
+    sketches on, also the count-min table and the HyperLogLog registers (fa_sketch_export)."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"flows": recs[record_order(recs)[:DUMP_FLOWS]].astype(np.float32),
+           "live_flows": np.array([len(recs)], dtype=np.float64)}
+    if sketch is not None:
+        out["cms"], out["hll"] = sketch[0].astype(np.float64), sketch[1].astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def oracle_flows(wl, first, n, chunk=1 << 22, sketch=None):
     """The oracle's flows for records [first, first+n) of the workload stream, sorted like record_order(); with `sketch`
     (the workload's sketch parameters) also the CPU restatement's count-min table and HLL registers over the same records."""
@@ -258,6 +277,8 @@ def run_ours(args, wl):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the engine has no CPU fallback)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs needs a single-GPU run")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -367,6 +388,13 @@ def run_ours(args, wl):
     value = world * B * args.steps / (total_ms / 1e3) / 1e6
     launches = st1["kernel_launches"] - st0["kernel_launches"]
     flows = eng.live_flows()
+    if args.dump_outputs:                            # the parity check below starts from an emptied table anyway
+        sk = None
+        if wl.get("sketch"):
+            sp = wl["sketch"]
+            sk = eng.sketch_export(sp["cms_log2_width"], sp["cms_depth"], sp["hll_precision"])
+        out_dev, nfl = evict_dev()
+        dump_outputs(args.dump_outputs, out_dev[: nfl * REC].cpu().numpy().reshape(-1, REC), sk)
     nvlink = agg.exchange_stats() if (world > 1 and hasattr(agg, "exchange_stats")) else None
     if nvlink is not None and getattr(agg, "profile", False):
         rounds_timed = args.steps * ((B + max_batch - 1) // max_batch)
@@ -737,7 +765,12 @@ def main():
                     help="N>1: 'peer' = K3 stores into the owners' buffers over NVLink (no host sync); 'nccl' = all_to_all_single")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-events", action="store_true", help="skip the 64-byte packet-event row of e2e")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the flows they left in the table (a key-hash sample of at most "
+                         f"{DUMP_FLOWS}) and, with sketches on, the sketch tables as DIR/<name>.npy (1 GPU, flow workloads)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "rttdns"):
+        ap.error("--dump-outputs covers the GPU arm of the flow workloads")
     if args.batch is None:
         args.batch = (3 << 26) if args.gpus == 1 else (1 << 27)
     if args.workload == "rttdns":

@@ -53,9 +53,10 @@ def _emulated_engine():
     L._lib = saved
 
 
-@pytest.fixture(scope="module")
+@pytest.fixture
 def engine_emul():
-    """The whole C ABI on the CPU (tests/emul/engine_emul.cpp) swapped in for libflowagg.so for one test module."""
+    """The whole C ABI on the CPU (tests/emul/engine_emul.cpp) swapped in for libflowagg.so for one test.  Not wider:
+    a module's `gpu` tests that run after its emulation tests must get the real library."""
     L, lib = _load_engine_emulation()
     saved, L._lib = L._lib, lib
     try:

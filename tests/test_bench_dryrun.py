@@ -191,6 +191,20 @@ def test_default_workload_is_the_10m_flow_headline(monkeypatch):
     assert line["parity_ok"]
 
 
+def test_dump_outputs_holds_what_the_timed_steps_folded(monkeypatch, tmp_path):
+    """--dump-outputs: the flows of warmup + --steps batches (all of them: they fit the sample), as float32 records;
+    the same arguments write the same files."""
+    argv = SMALL + ["--no-cpu", "--no-verify", "--no-e2e", "--steps", "2", "--warmup", "1"]
+    line, _ = run_bench(monkeypatch, 1, argv + ["--dump-outputs", str(tmp_path / "a")])
+    run_bench(monkeypatch, 1, argv + ["--dump-outputs", str(tmp_path / "b")])
+    flows = np.load(tmp_path / "a" / "flows.npy")
+    assert flows.dtype == np.float32 and flows.shape == (line["config"]["live_flows"], REC)
+    assert np.load(tmp_path / "a" / "live_flows.npy").tolist() == [line["config"]["live_flows"]]
+    assert np.array_equal(flows, np.load(tmp_path / "b" / "flows.npy"))
+    recs = np.ascontiguousarray(flows.astype(np.uint8)).view(O.REC_DTYPE).reshape(-1)
+    assert int(recs["packets"].sum()) == (1 + 2) * 8192
+
+
 @pytest.mark.parametrize("exchange", ["peer", "nccl"])
 def test_multi_gpu_line_and_matched_collectives(monkeypatch, exchange):
     line, dist = run_bench(monkeypatch, 2, SMALL + ["--gpus", "2", "--exchange", exchange])

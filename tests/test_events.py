@@ -72,6 +72,12 @@ def test_full_cut_with_events_on_the_emulation(engine_emul):
         assert np.array_equal(O.sort_records(a.evict()), O.sort_records(b.evict()))
 
 
+def test_the_gpu_tests_below_get_the_real_library():
+    """The emulation the tests above swapped in ends with them: the gpu tests of this module run on libflowagg.so."""
+    import netobserv_ebpf_agent_b200._lib as L
+    assert L.lib()._name == L.lib_path()
+
+
 @pytest.mark.gpu
 def test_events_gpu():
     check(n=400_000, n_keys=60_000, max_entries=1 << 17, max_batch=1 << 16)
