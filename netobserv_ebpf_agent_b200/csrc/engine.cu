@@ -3,11 +3,13 @@
 // There is NO CPU fallback: without a CUDA device fa_create fails with FA_E_NODEV.
 #include <cuda_runtime.h>
 
+#include <array>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <new>
@@ -102,6 +104,52 @@ ZipfTable* zipf_table(uint64_t n_keys, uint32_t s_milli) {
 }  // namespace
 
 // ------------------------------------------------------------------------ engine
+// Owner of one device (cudaMalloc) or pinned host (cudaHostAlloc) allocation; it converts to the raw pointer.
+// reserve(need, want) grows it: when it holds fewer than `need` bytes it frees the buffer and allocates max(need, want)
+// bytes, without copying the contents.
+template <class T, bool kPinned>
+class Buf {
+  public:
+    Buf() = default;
+    Buf(Buf&& o) noexcept { swap(o); }
+    Buf& operator=(Buf&& o) noexcept { swap(o); return *this; }
+    ~Buf() { reset(); }
+    cudaError_t reserve(size_t need, size_t want = 0) {
+        if (need <= bytes_) return cudaSuccess;
+        reset();
+        void* p = nullptr;
+        want = std::max(need, want);
+        const cudaError_t r = kPinned ? cudaHostAlloc(&p, want, cudaHostAllocDefault) : cudaMalloc(&p, want);
+        if (r == cudaSuccess) { p_ = static_cast<T*>(p); bytes_ = want; }
+        return r;
+    }
+    void swap(Buf& o) noexcept { std::swap(p_, o.p_); std::swap(bytes_, o.bytes_); }
+    T* get() const { return p_; }
+    operator T*() const { return p_; }
+    T* operator->() const { return p_; }
+
+  private:
+    void reset() {
+        if (p_) { if (kPinned) cudaFreeHost(p_); else cudaFree(p_); }
+        p_ = nullptr; bytes_ = 0;
+    }
+    T* p_ = nullptr;
+    size_t bytes_ = 0;
+};
+template <class T> using DevBuf = Buf<T, false>;
+template <class T> using PinnedBuf = Buf<T, true>;
+
+// The flow table's arrays.  Kernels take the plain fa::Table view by value.
+struct FlowTable {
+    DevBuf<uint4> ident, hot, feat_add, feat_dns, feat_drop;
+    DevBuf<uint32_t> occ;
+    uint64_t mask = 0;
+    fa::Table view() const { return {ident, hot, feat_add, feat_dns, feat_drop, occ, mask}; }
+    bool has_features() const { return feat_add || feat_dns || feat_drop; }
+};
+
+static uint64_t pow2_at_least(uint64_t p, uint64_t want) { while (p < want) p <<= 1; return p; }   // p: a power of two
+
 struct fa_engine {
     fa_config cfg{};
     int device = 0, sm_count = 148;
@@ -109,48 +157,48 @@ struct fa_engine {
     cudaStream_t copy_stream = nullptr;
     std::mutex mu;
 
-    fa::Table table{};
+    FlowTable table;
     uint64_t slots = 0, epoch = 0;
     // FA_F_NONBLOCKING_EVICT: a second, empty table.  fa_evict swaps the two under `mu` (the Accounter hands its map
     // over and goes on with a fresh one, pkg/flow/account.go:67-68,86-87) and scans the retired one on its own stream.
-    fa::Table table_spare{};
+    FlowTable table_spare;
     bool double_buffered = false;
     std::mutex evict_mu;                      // one eviction at a time (the reference's evictor is single-flight)
     cudaStream_t evict_stream = nullptr;
     cudaEvent_t ev_swap = nullptr;
-    fa::Counters* d_ctr_ev = nullptr;         // evict_out cursor of the scan of the retired table
-    unsigned long long* h_ev_out = nullptr;   // pinned
-    fa::Counters* d_ctr = nullptr;
-    fa::Counters* h_ctr = nullptr;            // pinned mirror
+    DevBuf<fa::Counters> d_ctr_ev;            // evict_out cursor of the scan of the retired table
+    PinnedBuf<unsigned long long> h_ev_out;
+    DevBuf<fa::Counters> d_ctr;
+    PinnedBuf<fa::Counters> h_ctr;            // mirror of d_ctr
     uint64_t max_batch = 0;
 
     // staging for host input (double buffered)
-    uint8_t* d_stage[2] = {nullptr, nullptr};
-    uint8_t* h_stage[2] = {nullptr, nullptr};
+    DevBuf<uint8_t> d_stage[2];
+    PinnedBuf<uint8_t> h_stage[2];
     cudaEvent_t ev_stage_free[2] = {nullptr, nullptr};   // kernel that consumed the stage finished
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};       // H2D copy into the stage finished
     int stage_cur = 0;
 
-    fa::FixupScratch* d_scratch = nullptr; uint32_t scratch_slots = 0;
-    uint32_t* d_spill_idx = nullptr;
-    uint32_t* d_cut_set = nullptr; uint32_t cut_set_slots = 0;
-    uint32_t* d_cut_bitmap = nullptr; uint32_t* d_cut_out = nullptr; uint32_t* h_cut_out = nullptr;
+    DevBuf<fa::FixupScratch> d_scratch; uint32_t scratch_slots = 0;
+    DevBuf<uint32_t> d_spill_idx;
+    DevBuf<uint32_t> d_cut_set; uint32_t cut_set_slots = 0;
+    DevBuf<uint32_t> d_cut_bitmap, d_cut_out; PinnedBuf<uint32_t> h_cut_out;
 
-    uint8_t* d_expanded = nullptr;            // ... and their 144-byte expansion (events handed in as device memory)
-    uint32_t* d_snap_src = nullptr;           // fa_ingest_snaps: snapshot index of every record parsed out of a chunk
-    uint32_t* d_snap_cnt = nullptr;           // ... records per CTA of the parse kernels, then the total + 3 filter counters (u64)
-    uint8_t* d_snap_verdict = nullptr;        // ... with a flow filter: keep / skip per snapshot of the chunk
+    DevBuf<uint8_t> d_expanded;               // 144-byte expansion of events, and records parsed out of snapshots
+    DevBuf<uint32_t> d_snap_src;              // fa_ingest_snaps: snapshot index of every record parsed out of a chunk
+    DevBuf<uint32_t> d_snap_cnt;              // ... records per CTA of the parse kernels, then the total + 3 filter counters (u64)
+    DevBuf<uint8_t> d_snap_verdict;           // ... with a flow filter: keep / skip per snapshot of the chunk
     fa::FilterSet filter{};                   // fa_set_flow_filter (n_rules == 0: no filter)
-    uint8_t* d_evict = nullptr; uint64_t evict_cap = 0;
-    uint8_t* d_evict_dns = nullptr; uint8_t* d_evict_add = nullptr; uint8_t* d_evict_present = nullptr;
-    uint32_t* d_slot_of_out = nullptr; uint64_t feat_evict_cap = 0;
-    uint32_t* d_slot_of = nullptr;            // per-sample slot scratch of the feature folds
+    DevBuf<uint8_t> d_evict;                  // eviction records for host memory, grown on demand
+    DevBuf<uint8_t> d_evict_dns, d_evict_add, d_evict_drop, d_evict_rttmin, d_evict_present;   // ... and its feature outputs
+    DevBuf<uint32_t> d_slot_of_out;
+    DevBuf<uint32_t> d_slot_of;               // per-sample slot scratch of the feature folds
     uint64_t feat_seq[3] = {0, 0, 0};         // running sample numbers (additional, dns, packet drops)
-    uint8_t* d_evict_drop = nullptr; unsigned long long* d_evict_rttmin = nullptr;
-    uint32_t* d_route_tmp = nullptr; unsigned long long* d_route_counts = nullptr;
+    DevBuf<uint32_t> d_route_tmp; DevBuf<unsigned long long> d_route_counts;
 
-    fa::SketchParams sk{};
-    unsigned long long* d_prof = nullptr;     // FA_PHASE_PROFILE=1: per-phase warp-cycle counters of K1
+    fa::SketchParams sk{};                    // cms / hll point into sk_cms / sk_hll
+    DevBuf<unsigned long long> sk_cms; DevBuf<uint32_t> sk_hll;
+    DevBuf<unsigned long long> d_prof;        // FA_PHASE_PROFILE=1: per-phase warp-cycle counters of K1
 #ifndef FA_K1_DEFAULT_OPT
 #define FA_K1_DEFAULT_OPT 0u                  // K1 switches an engine starts with (kernels.cuh, AggLaunch::opt); FA_K1_OPT overrides (diagnostics)
 #endif
@@ -161,33 +209,33 @@ struct fa_engine {
     uint64_t live_known = 0;
     uint64_t unsynced_records = 0;
     static constexpr int kLiveRing = 8;
-    unsigned long long* h_live_ring = nullptr;   // pinned, kLiveRing entries
+    PinnedBuf<unsigned long long> h_live_ring;   // kLiveRing entries
     cudaEvent_t ev_live[kLiveRing] = {};
     uint32_t ring_n[kLiveRing] = {};
     uint32_t ring_head = 0, ring_tail = 0;       // monotonically increasing; slot = idx % kLiveRing
 
     // KERNEL_MAP mode (kmap.cu): metrics lines, per-batch scratch, fallback ring
-    uint8_t* km_met = nullptr;
-    uint32_t* km_slot_of = nullptr;
-    fa::KmBEntry* km_bset = nullptr; uint32_t km_bset_slots = 0;
-    uint32_t* km_blist = nullptr;
-    uint32_t *km_touched = nullptr, *km_deferred = nullptr, *km_brec = nullptr;   // v2 work lists
+    DevBuf<uint8_t> km_met;
+    DevBuf<uint32_t> km_slot_of;
+    DevBuf<fa::KmBEntry> km_bset; uint32_t km_bset_slots = 0;
+    DevBuf<uint32_t> km_blist;
+    DevBuf<uint32_t> km_touched, km_deferred, km_brec;   // v2 work lists
     int km_impl = 2;                          // FA_KMAP_IMPL: 1 = seven per-record passes, 2 = per-flow finalisation
-    uint8_t* km_spill = nullptr; uint64_t km_spill_cap = 0;
-    fa::KmCounters* d_km_ctr = nullptr;
-    fa::KmCounters* h_km_ctr = nullptr;       // pinned mirror
+    DevBuf<uint8_t> km_spill; uint64_t km_spill_cap = 0;
+    DevBuf<fa::KmCounters> d_km_ctr;
+    PinnedBuf<fa::KmCounters> h_km_ctr;       // mirror of d_km_ctr
     uint64_t km_spilled_total = 0;            // records read back by fa_read_spilled so far
 
     // K8 scratch (fa_pb_encode), grown on demand
-    uint32_t* d_pb_sizes = nullptr; unsigned long long* d_pb_offsets = nullptr; unsigned long long* d_pb_sums = nullptr;
-    uint64_t pb_cap = 0;
-    fa::PbIface* d_pb_ifaces = nullptr; uint32_t pb_ifaces_cap = 0;
+    DevBuf<uint32_t> d_pb_sizes; DevBuf<unsigned long long> d_pb_offsets, d_pb_sums;
+    DevBuf<fa::PbIface> d_pb_ifaces;
 
     // K7 (dnscorr.cu): the dns_flows map + per-chunk scratch, allocated by the first fa_ingest_dns_packets
-    fa::DnsCorr dnsc{};                       // tab == nullptr until then
-    fa::DnsEntry* dnsc_spare = nullptr;       // the other table of a rebuild
-    unsigned long long* h_dnsc_ctr = nullptr; // pinned mirror of dnsc.ctr
-    uint32_t* d_dnsc_state = nullptr; uint8_t* d_dnsc_samples = nullptr; uint8_t* d_dnsc_out = nullptr; uint32_t* d_dnsc_warps = nullptr;
+    fa::DnsCorr dnsc{};                       // tab == nullptr until then; tab / ctr point into dnsc_tab / dnsc_ctr
+    DevBuf<fa::DnsEntry> dnsc_tab, dnsc_spare;   // the map, and the other table of a rebuild
+    DevBuf<unsigned long long> dnsc_ctr;
+    PinnedBuf<unsigned long long> h_dnsc_ctr; // mirror of dnsc_ctr
+    DevBuf<uint32_t> d_dnsc_state, d_dnsc_warps; DevBuf<uint8_t> d_dnsc_samples, d_dnsc_out;
     uint64_t dnsc_chunk = 0;                  // packets per launch_dns_correlate
     uint64_t dnsc_used = 0;                   // upper bound of the table entries in use (present + answered keys)
     uint64_t dnsc_slots = 0;                  // 4 x max_entries: answered keys keep their entry until the next rebuild
@@ -245,7 +293,7 @@ int launch_chunk(fa_engine* e, const uint8_t* d_recs, uint32_t n) {
     fa::AggLaunch a{};
     a.recs = reinterpret_cast<const uint4*>(d_recs);
     a.n = n;
-    a.table = e->table;
+    a.table = e->table.view();
     a.epoch = ++e->epoch;
     a.ctr = e->d_ctr;
     a.spill_idx = e->d_spill_idx;
@@ -258,6 +306,31 @@ int launch_chunk(fa_engine* e, const uint8_t* d_recs, uint32_t n) {
     e->st.kernel_launches += fa::launch_aggregate(a, e->stream);
     CU(cudaGetLastError());
     return note_launch(e, n);
+}
+
+// How many of the next n records to hand to a cache that may fill.  ACCOUNTER mode cuts a chunk after roughly `room`
+// new keys, so it gets a window proportional to the room left: the work stays linear in the records consumed however
+// small the cache is, and a "full" return does not leave most of a staged chunk unused (the caller hands the rest in
+// again after its eviction).  Other modes take all n.
+uint64_t room_window(fa_engine* e, uint64_t n) {
+    if (e->cfg.mode != FA_MODE_ACCOUNTER || (e->cfg.flags & FA_F_NO_FULL_CUT)) return n;
+    retire_completed(e);
+    const uint64_t used = e->live_known + e->unsynced_records;
+    const uint64_t room = e->cfg.max_entries > used ? e->cfg.max_entries - used : 0;
+    return std::min<uint64_t>(n, std::max<uint64_t>(4096, 4 * room));
+}
+
+// *cut = index of the first of the n records whose key is new while the cache holds max_entries flows (n: none).
+// e->live_known must be exact.
+int full_cut(fa_engine* e, const uint8_t* d_recs, uint32_t n, uint32_t* cut) {
+    e->st.kernel_launches += fa::launch_full_cut(reinterpret_cast<const uint4*>(d_recs), n, e->table.view(), e->live_known,
+                                                 e->cfg.max_entries, e->d_cut_set, e->cut_set_slots, e->d_cut_bitmap,
+                                                 e->d_cut_out, e->sm_count, e->stream);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(e->h_cut_out, e->d_cut_out, 4, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    *cut = *e->h_cut_out;
+    return FA_OK;
 }
 
 // ACCOUNTER mode: fold a device-resident chunk honouring max_entries.
@@ -289,19 +362,11 @@ int ingest_chunk_accounter(fa_engine* e, const uint8_t* d_recs, uint32_t n, uint
         *consumed = n;
         return FA_OK;
     }
-    // slow path: find the first record whose key is new while the cache is full.  The cut cannot come before `room`
-    // new keys have been seen, so it is looked for inside a window proportional to the room that is left: the pre-pass
-    // work stays linear in the records consumed however small the cache is.  A window without a cut is folded and the
-    // caller goes on with the rest of its chunk.
-    const uint64_t room = M > e->live_known ? M - e->live_known : 0;      // exact: the counters were just read
-    const uint32_t win = (uint32_t)std::min<uint64_t>(n, std::max<uint64_t>(4096, 4 * room));
-    e->st.kernel_launches += fa::launch_full_cut(reinterpret_cast<const uint4*>(d_recs), win, e->table, e->live_known, M,
-                                                 e->d_cut_set, e->cut_set_slots, e->d_cut_bitmap, e->d_cut_out,
-                                                 e->sm_count, e->stream);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(e->h_cut_out, e->d_cut_out, 4, cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    const uint32_t cut = *e->h_cut_out;
+    // slow path: find the first record whose key is new while the cache is full.  The counters were just read, so the
+    // room of the window is exact.  A window without a cut is folded and the caller goes on with the rest of its chunk.
+    const uint32_t win = (uint32_t)room_window(e, n);
+    uint32_t cut = 0;
+    if (int rc = full_cut(e, d_recs, win, &cut)) return rc;
     if (cut > 0) {
         int rc = launch_chunk(e, d_recs, cut);
         if (rc) return rc;
@@ -326,19 +391,13 @@ int ingest_chunk_kmap(fa_engine* e, const uint8_t* d_recs, uint32_t n, uint32_t*
     }
     uint32_t cut = n;                                  // records [cut, n) find the map full
     if (e->live_known + e->unsynced_records + n > M) {
-        e->st.kernel_launches += fa::launch_full_cut(reinterpret_cast<const uint4*>(d_recs), n, e->table, e->live_known, M,
-                                                     e->d_cut_set, e->cut_set_slots, e->d_cut_bitmap, e->d_cut_out,
-                                                     e->sm_count, e->stream);
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(e->h_cut_out, e->d_cut_out, 4, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaStreamSynchronize(e->stream));
-        cut = *e->h_cut_out;
+        if (int rc = full_cut(e, d_recs, n, &cut)) return rc;
         if (cut < n) e->st.full_cuts++;
     }
     fa::KmParams P{};
     P.recs = d_recs; P.n = n;
     P.ringbuf = (e->cfg.flags & FA_F_RINGBUF_FALLBACK) ? 1 : 0;
-    P.t = e->table; P.met = e->km_met;
+    P.t = e->table.view(); P.met = e->km_met;
     P.epoch = ++e->epoch;
     P.slot_of = e->km_slot_of;
     P.live = &e->d_ctr->live;
@@ -377,9 +436,10 @@ int ingest_device(fa_engine* e, const uint8_t* d_recs, size_t n, size_t* consume
 static uint64_t stage_records(const fa_engine* e) { return std::min<uint64_t>(e->max_batch, 1ull << 20); }   // 151 MB of records per copy
 
 static int stage_alloc(fa_engine* e, bool pageable) {
+    const size_t bytes = stage_records(e) * fa::kRecBytes;
     for (int i = 0; i < 2; i++) {
-        if (!e->d_stage[i]) CU(cudaMalloc(&e->d_stage[i], stage_records(e) * fa::kRecBytes));
-        if (pageable && !e->h_stage[i]) CU(cudaHostAlloc(&e->h_stage[i], stage_records(e) * fa::kRecBytes, cudaHostAllocDefault));
+        CU(e->d_stage[i].reserve(bytes));
+        if (pageable) CU(e->h_stage[i].reserve(bytes));
     }
     return FA_OK;
 }
@@ -402,45 +462,98 @@ static int stage_release(fa_engine* e, int sidx) {                   // the kern
     return FA_OK;
 }
 
-int ingest_host(fa_engine* e, const uint8_t* h_recs, size_t n, size_t* consumed, bool pinned) {
+// One chunk of caller memory as the device reads it: the caller's device memory in place, or a staging buffer.
+struct Chunk {
+    fa_engine* e;
+    const uint8_t* d;
+    int sidx;                                  // staging buffer, -1: none (or already released)
+    int release() {                            // the work enqueued so far was the chunk's last reader
+        const int s = sidx;
+        sidx = -1;
+        return s >= 0 ? stage_release(e, s) : FA_OK;
+    }
+};
+
+// Walks n items of `width` bytes of caller memory chunk by chunk.  Device memory (`align`-byte aligned) is read in
+// place; host memory goes through the staging buffers.  For each chunk, rule(left, staged, &c) sets its size c and may
+// enqueue work that has to come first; body(chunk, c, &took) enqueues the chunk's work, calls chunk.release() as soon
+// as the rest of that work no longer reads the chunk, and sets how many items it consumed.  The walk stops at the first
+// rule or body that does not return FA_OK.  The caller's buffer is not referenced after return.
+template <class Rule, class Body>
+int ingest_caller_memory(fa_engine* e, const char* who, const char* what, unsigned align, const void* src, size_t n,
+                         size_t width, size_t* consumed, Rule rule, Body body) {
+    const PtrKind k = classify(src);
+    if (k == PTR_DEVICE && (reinterpret_cast<uintptr_t>(src) & (align - 1)))
+        return fail(FA_E_INVAL, "%s: device %s must be %u-byte aligned", who, what, align);
+    const bool staged = k != PTR_DEVICE;
+    if (staged) { if (int rc = stage_alloc(e, k == PTR_PAGEABLE)) return rc; }
     size_t done = 0;
     int rc = FA_OK;
-    while (done < n) {
-        uint32_t c = (uint32_t)std::min<size_t>(n - done, stage_records(e));
-        if (e->cfg.mode == FA_MODE_ACCOUNTER && !(e->cfg.flags & FA_F_NO_FULL_CUT)) {
-            // A cache that is about to fill cuts the chunk after roughly `room` new keys: stage a window proportional
-            // to the room left, so that a "full" return does not leave most of a copied chunk unused (the caller
-            // hands the rest in again after its eviction).
-            retire_completed(e);
-            const uint64_t used = e->live_known + e->unsynced_records;
-            const uint64_t room = e->cfg.max_entries > used ? e->cfg.max_entries - used : 0;
-            if (room < c) c = (uint32_t)std::min<uint64_t>(c, std::max<uint64_t>(4096, 4 * room));
+    while (rc == FA_OK && done < n) {
+        size_t c = 0, took = 0;
+        if ((rc = rule(n - done, staged, &c))) break;
+        Chunk ch{e, static_cast<const uint8_t*>(src) + done * width, -1};
+        if (staged) {
+            if ((rc = stage_copy(e, ch.d, c * width, k == PTR_PINNED, &ch.sidx))) break;
+            ch.d = e->d_stage[ch.sidx];
         }
-        int sidx = 0;
-        if (int src_rc = stage_copy(e, h_recs + done * fa::kRecBytes, (size_t)c * fa::kRecBytes, pinned, &sidx)) return src_rc;
-        uint32_t off = 0;                                            // a chunk may be folded in several windows
-        while (off < c) {
-            uint32_t took = 0;
-            rc = ingest_chunk(e, e->d_stage[sidx] + (size_t)off * fa::kRecBytes, c - off, &took);
-            off += took;
-            if (rc != FA_OK) break;
-        }
-        if (int rel_rc = stage_release(e, sidx)) return rel_rc;
-        done += off;
-        if (rc != FA_OK) break;
+        rc = body(ch, c, &took);
+        if (int rel_rc = ch.release()) rc = rel_rc;
+        done += took;
     }
-    // the caller's buffer must not be referenced after return
-    CU(cudaStreamSynchronize(e->copy_stream));
     if (consumed) *consumed = done;
+    if (staged) CU(cudaStreamSynchronize(e->copy_stream));
     return rc;
 }
 
-}  // namespace
-
-static uint64_t e_max_batch_tmp(const fa_config* cfg) {
-    uint64_t mb = cfg->max_batch ? cfg->max_batch : (1ull << 22);
-    return mb > (1ull << 28) ? (1ull << 28) : mb;
+// Feature samples may create flows: never let the table pass 7/8 of its slots.
+int check_headroom(fa_engine* e, size_t n, const char* who, const char* what) {
+    if (int rc = sync_counters(e)) return rc;
+    if (e->live_known + n > e->slots - e->slots / 8)
+        return fail(FA_E_2BIG, "%s: %zu %s could overfill the flow table (%llu live of %llu slots): evict first", who, n, what,
+                    (unsigned long long)e->live_known, (unsigned long long)e->slots);
+    return FA_OK;
 }
+
+// Allocates `bytes` for b and zeroes them on the engine's stream.
+template <class T>
+int alloc_zeroed(fa_engine* e, DevBuf<T>& b, size_t bytes) {
+    CU(b.reserve(bytes));
+    CU(cudaMemsetAsync(b, 0, bytes, e->stream));
+    return FA_OK;
+}
+
+// fa_evict_out's optional per-flow outputs in the order they are copied back: the caller's pointer, the bytes per flow,
+// and the device buffer that stages the output when the caller's pointer is host memory.
+struct EvictOut { void* dst; size_t width; DevBuf<uint8_t>* stage; };
+using EvictOuts = std::array<EvictOut, 5>;
+EvictOuts evict_outputs(fa_engine* e, const fa_evict_out* o) {
+    return {{{o->dns, 64, &e->d_evict_dns}, {o->additional, 32, &e->d_evict_add}, {o->pkt_drops, 32, &e->d_evict_drop},
+             {o->rtt_min, 8, &e->d_evict_rttmin}, {o->present, 1, &e->d_evict_present}}};
+}
+
+// Grows an eviction buffer to `live` entries of `width` bytes, with room for twice as many (at most max_entries).
+template <class T>
+int reserve_evict(fa_engine* e, DevBuf<T>& b, uint64_t live, size_t width) {
+    CU(b.reserve(live * width, std::max<uint64_t>(live, std::min<uint64_t>(e->cfg.max_entries, live * 2)) * width));
+    return FA_OK;
+}
+
+// Where an eviction writes its records: the caller's device memory in place, else the engine's staging buffer.
+int evict_records_dst(fa_engine* e, void* records, uint64_t live, uint8_t** d_out) {
+    if (classify(records) == PTR_DEVICE) { *d_out = static_cast<uint8_t*>(records); return FA_OK; }
+    if (int rc = reserve_evict(e, e->d_evict, live, fa::kRecBytes)) return rc;
+    *d_out = e->d_evict;
+    return FA_OK;
+}
+
+// Without feature tables, the feature outputs in host memory come back zeroed.
+void zero_host_outputs(const EvictOuts& outs, uint64_t live) {
+    for (const EvictOut& x : outs)
+        if (x.dst && classify(x.dst) != PTR_DEVICE) memset(x.dst, 0, live * x.width);
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -476,104 +589,76 @@ int fa_create(const fa_config* cfg, fa_engine** out) {
     e->cfg = *cfg;
     e->device = cfg->device;
     e->sm_count = prop.multiProcessorCount;
-    e->max_batch = cfg->max_batch ? cfg->max_batch : (1ull << 22);
-    if (e->max_batch > (1ull << 28)) e->max_batch = 1ull << 28;
+    e->max_batch = std::min<uint64_t>(cfg->max_batch ? cfg->max_batch : (1ull << 22), 1ull << 28);
     if (cfg->cuda_stream) { e->stream = (cudaStream_t)cfg->cuda_stream; }
     else { CU(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking)); e->own_stream = true; }
     CU(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
 
     // table: load factor <= 0.75 at max_entries
-    uint64_t want = (4 * cfg->max_entries + 2) / 3;          // 0.75 x 2^k entries get exactly 2^k slots
-    uint64_t slots = 1024; while (slots < want) slots <<= 1;
+    const uint64_t slots = pow2_at_least(1024, (4 * cfg->max_entries + 2) / 3);   // 0.75 x 2^k entries get exactly 2^k slots
     e->slots = slots;
     e->table.mask = slots - 1;
-    CU(cudaMalloc(&e->table.ident, slots * fa::kIdentBytes));
-    CU(cudaMemsetAsync(e->table.ident, 0, slots * fa::kIdentBytes, e->stream));
+    if (int rc = alloc_zeroed(e, e->table.ident, slots * fa::kIdentBytes)) return rc;
     if (!kmap) {
-        CU(cudaMalloc(&e->table.hot, slots * fa::kHotBytes));
-        CU(cudaMemsetAsync(e->table.hot, 0, slots * fa::kHotBytes, e->stream));
+        if (int rc = alloc_zeroed(e, e->table.hot, slots * fa::kHotBytes)) return rc;
     } else {
         if (slots > (1ull << 30)) return fail(FA_E_INVAL, "fa_create: KERNEL_MAP mode supports at most 2^30 slots");
-        CU(cudaMalloc(&e->km_met, slots * fa::kMetLineBytes));
-        CU(cudaMemsetAsync(e->km_met, 0, slots * fa::kMetLineBytes, e->stream));
-        CU(cudaMalloc(&e->km_slot_of, e->max_batch * 4));
-        uint32_t bs = 1024; while ((uint64_t)bs < 2 * e->max_batch) bs <<= 1;
-        e->km_bset_slots = bs;
-        CU(cudaMalloc(&e->km_bset, (size_t)bs * sizeof(fa::KmBEntry)));
-        CU(cudaMemsetAsync(e->km_bset, 0, (size_t)bs * sizeof(fa::KmBEntry), e->stream));
-        CU(cudaMalloc(&e->km_blist, e->max_batch * 4));
-        CU(cudaMalloc(&e->km_touched, e->max_batch * 4));
-        CU(cudaMalloc(&e->km_deferred, e->max_batch * 4));
-        CU(cudaMalloc(&e->km_brec, e->max_batch * 4));
+        if (int rc = alloc_zeroed(e, e->km_met, slots * fa::kMetLineBytes)) return rc;
+        CU(e->km_slot_of.reserve(e->max_batch * 4));
+        e->km_bset_slots = (uint32_t)pow2_at_least(1024, 2 * e->max_batch);
+        if (int rc = alloc_zeroed(e, e->km_bset, (size_t)e->km_bset_slots * sizeof(fa::KmBEntry))) return rc;
+        CU(e->km_blist.reserve(e->max_batch * 4));
+        CU(e->km_touched.reserve(e->max_batch * 4));
+        CU(e->km_deferred.reserve(e->max_batch * 4));
+        CU(e->km_brec.reserve(e->max_batch * 4));
         if (const char* ki = getenv("FA_KMAP_IMPL")) e->km_impl = ki[0] == '1' ? 1 : 2;
         if (cfg->flags & FA_F_RINGBUF_FALLBACK) {
             e->km_spill_cap = 131072;                   // >= the 16 MiB direct_flows ring (bpf/maps_definition.h:7-11)
-            CU(cudaMalloc(&e->km_spill, e->km_spill_cap * fa::kRecBytes));
+            CU(e->km_spill.reserve(e->km_spill_cap * fa::kRecBytes));
         }
-        CU(cudaMalloc(&e->d_km_ctr, sizeof(fa::KmCounters)));
-        CU(cudaMemsetAsync(e->d_km_ctr, 0, sizeof(fa::KmCounters), e->stream));
-        CU(cudaHostAlloc(&e->h_km_ctr, sizeof(fa::KmCounters), cudaHostAllocDefault));
+        if (int rc = alloc_zeroed(e, e->d_km_ctr, sizeof(fa::KmCounters))) return rc;
+        CU(e->h_km_ctr.reserve(sizeof(fa::KmCounters)));
         memset(e->h_km_ctr, 0, sizeof(fa::KmCounters));
     }
-    CU(cudaMalloc(&e->table.occ, slots / 8));
-    CU(cudaMemsetAsync(e->table.occ, 0, slots / 8, e->stream));
+    if (int rc = alloc_zeroed(e, e->table.occ, slots / 8)) return rc;
     if (cfg->flags & FA_F_NONBLOCKING_EVICT) {
         if (kmap || (cfg->flags & (FA_F_ENABLE_RTT | FA_F_ENABLE_DNS | FA_F_ENABLE_PKT_DROP)))
             return fail(FA_E_INVAL, "fa_create: FA_F_NONBLOCKING_EVICT is available in ACCOUNTER mode without feature folds");
         e->table_spare.mask = slots - 1;
-        CU(cudaMalloc(&e->table_spare.ident, slots * fa::kIdentBytes));
-        CU(cudaMemsetAsync(e->table_spare.ident, 0, slots * fa::kIdentBytes, e->stream));
-        CU(cudaMalloc(&e->table_spare.hot, slots * fa::kHotBytes));
-        CU(cudaMemsetAsync(e->table_spare.hot, 0, slots * fa::kHotBytes, e->stream));
-        CU(cudaMalloc(&e->table_spare.occ, slots / 8));
-        CU(cudaMemsetAsync(e->table_spare.occ, 0, slots / 8, e->stream));
+        if (int rc = alloc_zeroed(e, e->table_spare.ident, slots * fa::kIdentBytes)) return rc;
+        if (int rc = alloc_zeroed(e, e->table_spare.hot, slots * fa::kHotBytes)) return rc;
+        if (int rc = alloc_zeroed(e, e->table_spare.occ, slots / 8)) return rc;
         CU(cudaStreamCreateWithFlags(&e->evict_stream, cudaStreamNonBlocking));
         CU(cudaEventCreateWithFlags(&e->ev_swap, cudaEventDisableTiming));
-        CU(cudaMalloc(&e->d_ctr_ev, sizeof(fa::Counters)));
-        CU(cudaMemsetAsync(e->d_ctr_ev, 0, sizeof(fa::Counters), e->stream));
-        CU(cudaHostAlloc(&e->h_ev_out, 8, cudaHostAllocDefault));
+        if (int rc = alloc_zeroed(e, e->d_ctr_ev, sizeof(fa::Counters))) return rc;
+        CU(e->h_ev_out.reserve(8));
         e->double_buffered = true;
     }
-    if (cfg->flags & FA_F_ENABLE_RTT) {
-        CU(cudaMalloc(&e->table.feat_add, slots * 80));
-        CU(cudaMemsetAsync(e->table.feat_add, 0, slots * 80, e->stream));
-    }
-    if (cfg->flags & FA_F_ENABLE_DNS) {
-        CU(cudaMalloc(&e->table.feat_dns, slots * 128));
-        CU(cudaMemsetAsync(e->table.feat_dns, 0, slots * 128, e->stream));
-    }
-    if (cfg->flags & FA_F_ENABLE_PKT_DROP) {
-        CU(cudaMalloc(&e->table.feat_drop, slots * 96));
-        CU(cudaMemsetAsync(e->table.feat_drop, 0, slots * 96, e->stream));
-    }
-    if (cfg->flags & (FA_F_ENABLE_RTT | FA_F_ENABLE_DNS | FA_F_ENABLE_PKT_DROP)) CU(cudaMalloc(&e->d_slot_of, e_max_batch_tmp(cfg) * 4));
-    CU(cudaMalloc(&e->d_ctr, sizeof(fa::Counters)));
-    CU(cudaMemsetAsync(e->d_ctr, 0, sizeof(fa::Counters), e->stream));
-    CU(cudaHostAlloc(&e->h_ctr, sizeof(fa::Counters), cudaHostAllocDefault));
+    if (cfg->flags & FA_F_ENABLE_RTT) { if (int rc = alloc_zeroed(e, e->table.feat_add, slots * 80)) return rc; }
+    if (cfg->flags & FA_F_ENABLE_DNS) { if (int rc = alloc_zeroed(e, e->table.feat_dns, slots * 128)) return rc; }
+    if (cfg->flags & FA_F_ENABLE_PKT_DROP) { if (int rc = alloc_zeroed(e, e->table.feat_drop, slots * 96)) return rc; }
+    if (cfg->flags & (FA_F_ENABLE_RTT | FA_F_ENABLE_DNS | FA_F_ENABLE_PKT_DROP)) CU(e->d_slot_of.reserve(e->max_batch * 4));
+    if (int rc = alloc_zeroed(e, e->d_ctr, sizeof(fa::Counters))) return rc;
+    CU(e->h_ctr.reserve(sizeof(fa::Counters)));
     memset(e->h_ctr, 0, sizeof(fa::Counters));
-    CU(cudaHostAlloc(&e->h_live_ring, fa_engine::kLiveRing * 8, cudaHostAllocDefault));
+    CU(e->h_live_ring.reserve(fa_engine::kLiveRing * 8));
     for (int i = 0; i < fa_engine::kLiveRing; i++) CU(cudaEventCreateWithFlags(&e->ev_live[i], cudaEventDisableTiming));
 
     for (int i = 0; i < 2; i++) {
         CU(cudaEventCreateWithFlags(&e->ev_stage_free[i], cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&e->ev_copied[i], cudaEventDisableTiming));
     }
-    {
-        // one entry per flow that needs the ordered re-fold in a launch: at most one per record, and never more than the
-        // table has slots (entries are keyed by table slot)
-        uint32_t ss = 1024; while ((uint64_t)ss < 2 * std::min<uint64_t>(e->max_batch, e->slots)) ss <<= 1;
-        e->scratch_slots = ss;
-        CU(cudaMalloc(&e->d_scratch, (size_t)ss * sizeof(fa::FixupScratch)));
-        CU(cudaMemsetAsync(e->d_scratch, 0, (size_t)ss * sizeof(fa::FixupScratch), e->stream));
-        CU(cudaStreamSynchronize(e->stream));
-    }
-    CU(cudaMalloc(&e->d_spill_idx, e->max_batch * sizeof(uint32_t)));
-    uint32_t cs = 1024; while ((uint64_t)cs < 2 * e->max_batch) cs <<= 1;
-    e->cut_set_slots = cs;
-    CU(cudaMalloc(&e->d_cut_set, (size_t)cs * 4));
-    CU(cudaMalloc(&e->d_cut_bitmap, (e->max_batch + 31) / 32 * 4 + 4));
-    CU(cudaMalloc(&e->d_cut_out, 4));
-    CU(cudaHostAlloc(&e->h_cut_out, 4, cudaHostAllocDefault));
+    // one entry per flow that needs the ordered re-fold in a launch: at most one per record, and never more than the
+    // table has slots (entries are keyed by table slot)
+    e->scratch_slots = (uint32_t)pow2_at_least(1024, 2 * std::min<uint64_t>(e->max_batch, e->slots));
+    if (int rc = alloc_zeroed(e, e->d_scratch, (size_t)e->scratch_slots * sizeof(fa::FixupScratch))) return rc;
+    CU(cudaStreamSynchronize(e->stream));
+    CU(e->d_spill_idx.reserve(e->max_batch * sizeof(uint32_t)));
+    e->cut_set_slots = (uint32_t)pow2_at_least(1024, 2 * e->max_batch);
+    CU(e->d_cut_set.reserve((size_t)e->cut_set_slots * 4));
+    CU(e->d_cut_bitmap.reserve((e->max_batch + 31) / 32 * 4 + 4));
+    CU(e->d_cut_out.reserve(4));
+    CU(e->h_cut_out.reserve(4));
 
     // sketches
     e->sk.log2w = cfg->cms_log2_width ? cfg->cms_log2_width : 20;
@@ -583,15 +668,13 @@ int fa_create(const fa_config* cfg, fa_engine** out) {
     if (e->sk.depth > 8 || e->sk.log2w < 4 || e->sk.log2w > 30 || e->sk.p < 4 || e->sk.p > 18)
         return fail(FA_E_INVAL, "fa_create: sketch parameters out of range");
     if (cfg->flags & FA_F_ENABLE_SKETCH) {
-        const size_t cms_bytes = ((size_t)e->sk.depth << e->sk.log2w) * 8;
-        CU(cudaMalloc(&e->sk.cms, cms_bytes));
-        CU(cudaMemsetAsync(e->sk.cms, 0, cms_bytes, e->stream));
-        CU(cudaMalloc(&e->sk.hll, ((size_t)1 << e->sk.p) * 4));
-        CU(cudaMemsetAsync(e->sk.hll, 0, ((size_t)1 << e->sk.p) * 4, e->stream));
+        if (int rc = alloc_zeroed(e, e->sk_cms, ((size_t)e->sk.depth << e->sk.log2w) * 8)) return rc;
+        if (int rc = alloc_zeroed(e, e->sk_hll, ((size_t)1 << e->sk.p) * 4)) return rc;
+        e->sk.cms = e->sk_cms; e->sk.hll = e->sk_hll;
     }
     if (const char* ko = getenv("FA_K1_OPT")) e->k1_opt = (uint32_t)strtoul(ko, nullptr, 0);
     if (const char* pp = getenv("FA_PHASE_PROFILE")) {
-        if (pp[0] == '1') { CU(cudaMalloc(&e->d_prof, 16 * 8)); CU(cudaMemsetAsync(e->d_prof, 0, 128, e->stream)); }
+        if (pp[0] == '1') { if (int rc = alloc_zeroed(e, e->d_prof, 16 * 8)) return rc; }
     }
     CU(cudaStreamSynchronize(e->stream));
     guard.e = nullptr;
@@ -602,7 +685,7 @@ int fa_create(const fa_config* cfg, fa_engine** out) {
 void fa_destroy(fa_engine* e) {
     if (!e) return;
     cudaSetDevice(e->device);
-    if (e->stream) cudaStreamSynchronize(e->stream);
+    for (cudaStream_t s : {e->stream, e->copy_stream, e->evict_stream}) if (s) cudaStreamSynchronize(s);
     if (e->d_prof) {
         unsigned long long p[16];
         if (cudaMemcpy(p, e->d_prof, 128, cudaMemcpyDeviceToHost) == cudaSuccess) {
@@ -618,37 +701,11 @@ void fa_destroy(fa_engine* e) {
                     100.0 * p[10] / (double)std::max<uint64_t>(1, e->st.records_ingested), p[11]);
             fprintf(stderr, "[flowagg] K1 probes: home-slot collisions %llu, resolved one slot on %llu, unsettled at first probe %llu\n", p[12], p[13], p[14]);
         }
-        cudaFree(e->d_prof);
     }
-    if (e->copy_stream) { cudaStreamSynchronize(e->copy_stream); cudaStreamDestroy(e->copy_stream); }
-    if (e->evict_stream) { cudaStreamSynchronize(e->evict_stream); cudaStreamDestroy(e->evict_stream); }
-    if (e->ev_swap) cudaEventDestroy(e->ev_swap);
-    cudaFree(e->table_spare.ident); cudaFree(e->table_spare.hot); cudaFree(e->table_spare.occ); cudaFree(e->d_ctr_ev);
-    if (e->h_ev_out) cudaFreeHost(e->h_ev_out);
-    cudaFree(e->table.ident); cudaFree(e->table.hot); cudaFree(e->table.occ); cudaFree(e->table.feat_add); cudaFree(e->table.feat_dns); cudaFree(e->table.feat_drop);
-    cudaFree(e->d_ctr); if (e->h_ctr) cudaFreeHost(e->h_ctr);
-    if (e->h_live_ring) cudaFreeHost(e->h_live_ring);
-    for (int i = 0; i < fa_engine::kLiveRing; i++) if (e->ev_live[i]) cudaEventDestroy(e->ev_live[i]);
-    for (int i = 0; i < 2; i++) {
-        cudaFree(e->d_stage[i]); if (e->h_stage[i]) cudaFreeHost(e->h_stage[i]);
-        if (e->ev_stage_free[i]) cudaEventDestroy(e->ev_stage_free[i]);
-        if (e->ev_copied[i]) cudaEventDestroy(e->ev_copied[i]);
-    }
-    cudaFree(e->d_scratch); cudaFree(e->d_spill_idx); cudaFree(e->d_cut_set); cudaFree(e->d_cut_bitmap); cudaFree(e->d_cut_out);
-    if (e->h_cut_out) cudaFreeHost(e->h_cut_out);
-    cudaFree(e->d_evict); cudaFree(e->d_route_tmp); cudaFree(e->d_route_counts); cudaFree(e->d_expanded);
-    cudaFree(e->d_snap_src); cudaFree(e->d_snap_cnt); cudaFree(e->d_snap_verdict);
-    cudaFree(e->d_evict_dns); cudaFree(e->d_evict_add); cudaFree(e->d_evict_present); cudaFree(e->d_slot_of_out); cudaFree(e->d_slot_of);
-    cudaFree(e->d_evict_drop); cudaFree(e->d_evict_rttmin);
-    cudaFree(e->sk.cms); cudaFree(e->sk.hll);
-    cudaFree(e->dnsc.tab); cudaFree(e->dnsc_spare); cudaFree(e->dnsc.ctr); cudaFreeHost(e->h_dnsc_ctr);
-    cudaFree(e->d_dnsc_state); cudaFree(e->d_dnsc_samples); cudaFree(e->d_dnsc_out); cudaFree(e->d_dnsc_warps);
-    cudaFree(e->km_met); cudaFree(e->km_slot_of); cudaFree(e->km_bset); cudaFree(e->km_blist); cudaFree(e->km_spill);
-    cudaFree(e->km_touched); cudaFree(e->km_deferred); cudaFree(e->km_brec);
-    cudaFree(e->d_km_ctr); if (e->h_km_ctr) cudaFreeHost(e->h_km_ctr);
-    cudaFree(e->d_pb_sizes); cudaFree(e->d_pb_offsets); cudaFree(e->d_pb_sums); cudaFree(e->d_pb_ifaces);
-    if (e->own_stream && e->stream) cudaStreamDestroy(e->stream);
-    delete e;
+    for (cudaStream_t s : {e->copy_stream, e->evict_stream, e->own_stream ? e->stream : nullptr}) if (s) cudaStreamDestroy(s);
+    for (cudaEvent_t ev : e->ev_live) if (ev) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : {e->ev_swap, e->ev_stage_free[0], e->ev_stage_free[1], e->ev_copied[0], e->ev_copied[1]}) if (ev) cudaEventDestroy(ev);
+    delete e;                                         // the buffers free themselves
 }
 
 int fa_ingest(fa_engine* e, const void* recs, size_t n, size_t* consumed) {
@@ -658,13 +715,14 @@ int fa_ingest(fa_engine* e, const void* recs, size_t n, size_t* consumed) {
     if (!recs) return fail(FA_E_INVAL, "fa_ingest: null records");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    const PtrKind k = classify(recs);
-    if (k == PTR_DEVICE) {
-        if (reinterpret_cast<uintptr_t>(recs) & 15) return fail(FA_E_INVAL, "fa_ingest: device records must be 16-byte aligned");
-        return ingest_device(e, static_cast<const uint8_t*>(recs), n, consumed);
-    }
-    if (int rc = stage_alloc(e, k == PTR_PAGEABLE)) return rc;
-    return ingest_host(e, static_cast<const uint8_t*>(recs), n, consumed, k == PTR_PINNED);
+    // device records are folded in place, host records as their chunks are staged
+    return ingest_caller_memory(
+        e, "fa_ingest", "records", 16, recs, n, fa::kRecBytes, consumed,
+        [&](size_t left, bool staged, size_t* c) {
+            *c = staged ? room_window(e, std::min<uint64_t>(left, stage_records(e))) : left;
+            return FA_OK;
+        },
+        [&](Chunk& ch, size_t c, size_t* took) { return ingest_device(e, ch.d, c, took); });
 }
 
 int fa_ingest_events(fa_engine* e, const void* events, size_t n, size_t* consumed) {
@@ -675,45 +733,21 @@ int fa_ingest_events(fa_engine* e, const void* events, size_t n, size_t* consume
     static_assert(sizeof(fa_packet_event) == 64, "fa_packet_event ABI");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    const PtrKind k = classify(events);
-    if (k == PTR_DEVICE && (reinterpret_cast<uintptr_t>(events) & 15)) return fail(FA_E_INVAL, "fa_ingest_events: device events must be 16-byte aligned");
-    if (!e->d_expanded) CU(cudaMalloc(&e->d_expanded, e->max_batch * fa::kRecBytes));
-    if (k != PTR_DEVICE) { if (int arc = stage_alloc(e, k == PTR_PAGEABLE)) return arc; }
-    size_t done = 0;
-    int rc = FA_OK;
-    while (done < n) {
-        uint32_t c = (uint32_t)std::min<size_t>(n - done, k == PTR_DEVICE ? e->max_batch : stage_records(e));
-        if (e->cfg.mode == FA_MODE_ACCOUNTER && !(e->cfg.flags & FA_F_NO_FULL_CUT)) {     // see ingest_host: stage by the room left
-            retire_completed(e);
-            const uint64_t used = e->live_known + e->unsynced_records;
-            const uint64_t room = e->cfg.max_entries > used ? e->cfg.max_entries - used : 0;
-            if (room < c) c = (uint32_t)std::min<uint64_t>(c, std::max<uint64_t>(4096, 4 * room));
-        }
-        const uint8_t* src = static_cast<const uint8_t*>(events) + done * 64;
-        const uint8_t* d_ev = src;
-        // host events: staged like fa_ingest's records (the copy of the next chunk overlaps this chunk's kernels); the
-        // expansion and K1 of successive chunks are ordered on the engine's stream, so one d_expanded is enough
-        int sidx = -1;
-        if (k != PTR_DEVICE) {
-            if (int src_rc = stage_copy(e, src, (size_t)c * 64, k == PTR_PINNED, &sidx)) return src_rc;
-            d_ev = e->d_stage[sidx];
-        }
-        e->st.kernel_launches += fa::launch_expand_events(reinterpret_cast<const uint4*>(d_ev), c, reinterpret_cast<uint4*>(e->d_expanded), e->stream);
-        CU(cudaGetLastError());
-        if (sidx >= 0) { if (int rel_rc = stage_release(e, sidx)) return rel_rc; }
-        uint32_t off = 0;
-        while (off < c) {                                   // a chunk may be folded in several windows ("full" cuts)
-            uint32_t took = 0;
-            rc = ingest_chunk(e, e->d_expanded + (size_t)off * fa::kRecBytes, c - off, &took);
-            off += took;
-            if (rc != FA_OK) break;
-        }
-        done += off;
-        if (rc != FA_OK) break;
-    }
-    if (k != PTR_DEVICE) CU(cudaStreamSynchronize(e->copy_stream));   // the caller's buffer must not be referenced after return
-    if (consumed) *consumed = done;
-    return rc;
+    CU(e->d_expanded.reserve(e->max_batch * fa::kRecBytes));
+    // the expansion and K1 of successive chunks are ordered on the engine's stream, so one d_expanded is enough
+    return ingest_caller_memory(
+        e, "fa_ingest_events", "events", 16, events, n, 64, consumed,
+        [&](size_t left, bool staged, size_t* c) {
+            *c = room_window(e, std::min<uint64_t>(left, staged ? stage_records(e) : e->max_batch));
+            return FA_OK;
+        },
+        [&](Chunk& ch, size_t c, size_t* took) {
+            e->st.kernel_launches += fa::launch_expand_events(reinterpret_cast<const uint4*>(ch.d), (uint32_t)c,
+                                                              reinterpret_cast<uint4*>(e->d_expanded.get()), e->stream);
+            CU(cudaGetLastError());
+            if (int rc = ch.release()) return rc;
+            return ingest_device(e, e->d_expanded, c, took);   // a chunk may be folded in several windows ("full" cuts)
+        });
 }
 
 int fa_ingest_snaps(fa_engine* e, const void* snaps, size_t n, uint32_t stride, size_t* consumed) {
@@ -724,68 +758,53 @@ int fa_ingest_snaps(fa_engine* e, const void* snaps, size_t n, uint32_t stride, 
     if (!snaps) return fail(FA_E_INVAL, "fa_ingest_snaps: null snapshots");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    const PtrKind k = classify(snaps);
-    if (k == PTR_DEVICE && (reinterpret_cast<uintptr_t>(snaps) & 7)) return fail(FA_E_INVAL, "fa_ingest_snaps: device snapshots must be 8-byte aligned");
-    if (!e->d_expanded) CU(cudaMalloc(&e->d_expanded, e->max_batch * fa::kRecBytes));
-    if (!e->d_snap_src) CU(cudaMalloc(&e->d_snap_src, e->max_batch * sizeof(uint32_t)));
-    if (!e->d_snap_cnt) CU(cudaMalloc(&e->d_snap_cnt, (fa::kSnapMaxCtas + 8) * sizeof(uint32_t)));
-    if (e->filter.n_rules && !e->d_snap_verdict) CU(cudaMalloc(&e->d_snap_verdict, e->max_batch));
-    if (k != PTR_DEVICE) { if (int arc = stage_alloc(e, k == PTR_PAGEABLE)) return arc; }
-    unsigned long long* d_total = reinterpret_cast<unsigned long long*>(e->d_snap_cnt + fa::kSnapMaxCtas);
-    // host chunks are bounded by the staging buffers (stage_records() x 144 bytes), device chunks by max_batch records
-    const size_t per_chunk = k == PTR_DEVICE ? e->max_batch : std::min<uint64_t>(e->max_batch, stage_records(e) * fa::kRecBytes / stride);
-    size_t done = 0;
-    int rc = FA_OK;
-    while (done < n) {
-        const uint32_t c = (uint32_t)std::min<size_t>(n - done, per_chunk);
-        const uint8_t* src = static_cast<const uint8_t*>(snaps) + done * stride;
-        const uint8_t* d_sn = src;
-        int sidx = -1;
-        if (k != PTR_DEVICE) {
-            if (int src_rc = stage_copy(e, src, (size_t)c * stride, k == PTR_PINNED, &sidx)) return src_rc;
-            d_sn = e->d_stage[sidx];
-        }
-        CU(cudaMemsetAsync(d_total + 1, 0, 24, e->stream));             // the filter's three counters of this chunk
-        e->st.kernel_launches += fa::launch_parse_snaps(d_sn, c, stride, &e->filter, e->d_snap_cnt, e->d_snap_verdict,
-                                                        reinterpret_cast<uint4*>(e->d_expanded), e->d_snap_src, d_total, d_total + 1,
-                                                        e->sm_count, e->stream);
-        CU(cudaGetLastError());
-        if (sidx >= 0) { if (int rel_rc = stage_release(e, sidx)) return rel_rc; }
-        // how many packets were submitted decides the launch sizes of the fold: one 8-byte read-back per chunk
-        unsigned long long back[4] = {0, 0, 0, 0};                      // submitted + kept | filter accept / reject / no match
-        CU(cudaMemcpyAsync(back, d_total, 32, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaStreamSynchronize(e->stream));
-        const uint32_t m = (uint32_t)back[0];
-        e->st.filter_accept += back[1]; e->st.filter_reject += back[2]; e->st.filter_nomatch += back[3];
-        // every submitted packet bumps exactly one of the three counters: what the filter skipped = submitted - kept
-        const uint64_t filtered_out = e->filter.n_rules ? back[1] + back[2] + back[3] - (uint64_t)m : 0;
-        uint32_t off = 0;
-        while (off < m) {                                   // a chunk may be folded in several windows ("full" cuts)
-            uint32_t took = 0;
-            rc = ingest_chunk(e, e->d_expanded + (size_t)off * fa::kRecBytes, m - off, &took);
-            off += took;
-            if (rc != FA_OK) break;
-        }
-        if (rc == FA_FULL && off < m) {
-            // the cut is reported in snapshots: everything before the first record that was not folded, discarded ones included
-            uint32_t first_left = 0;
-            CU(cudaMemcpyAsync(&first_left, e->d_snap_src + off, 4, cudaMemcpyDeviceToHost, e->stream));
+    CU(e->d_expanded.reserve(e->max_batch * fa::kRecBytes));
+    CU(e->d_snap_src.reserve(e->max_batch * sizeof(uint32_t)));
+    CU(e->d_snap_cnt.reserve((fa::kSnapMaxCtas + 8) * sizeof(uint32_t)));
+    if (e->filter.n_rules) CU(e->d_snap_verdict.reserve(e->max_batch));
+    unsigned long long* d_total = reinterpret_cast<unsigned long long*>(e->d_snap_cnt.get() + fa::kSnapMaxCtas);
+    return ingest_caller_memory(
+        e, "fa_ingest_snaps", "snapshots", 8, snaps, n, stride, consumed,
+        [&](size_t left, bool staged, size_t* c) {
+            // host chunks are bounded by the staging buffers (stage_records() x 144 bytes), device chunks by max_batch records
+            *c = std::min<uint64_t>(left, staged ? std::min<uint64_t>(e->max_batch, stage_records(e) * fa::kRecBytes / stride) : e->max_batch);
+            return FA_OK;
+        },
+        [&](Chunk& ch, size_t c, size_t* took) {
+            CU(cudaMemsetAsync(d_total + 1, 0, 24, e->stream));             // the filter's three counters of this chunk
+            e->st.kernel_launches += fa::launch_parse_snaps(ch.d, (uint32_t)c, stride, &e->filter, e->d_snap_cnt, e->d_snap_verdict,
+                                                            reinterpret_cast<uint4*>(e->d_expanded.get()), e->d_snap_src, d_total,
+                                                            d_total + 1, e->sm_count, e->stream);
+            CU(cudaGetLastError());
+            if (int rc = ch.release()) return rc;
+            // how many packets were submitted decides the launch sizes of the fold: one 8-byte read-back per chunk
+            unsigned long long back[4] = {0, 0, 0, 0};                      // submitted + kept | filter accept / reject / no match
+            CU(cudaMemcpyAsync(back, d_total, 32, cudaMemcpyDeviceToHost, e->stream));
             CU(cudaStreamSynchronize(e->stream));
-            // discarded snapshots before the cut: first_left - off
-            // (with a filter the discarded / filtered split of a partially consumed chunk is not known: both count as discarded)
-            e->st.snaps_ingested += first_left;
-            e->st.snaps_discarded += first_left - off;
-            done += first_left;
-            break;
-        }
-        if (rc != FA_OK) break;
-        e->st.snaps_ingested += c;
-        e->st.snaps_discarded += c - m - filtered_out;                  // fill_ethhdr's DISCARDs; the filter's skips are in its counters
-        done += c;
-    }
-    if (k != PTR_DEVICE) CU(cudaStreamSynchronize(e->copy_stream));   // the caller's buffer must not be referenced after return
-    if (consumed) *consumed = done;
-    return rc;
+            const uint32_t m = (uint32_t)back[0];
+            e->st.filter_accept += back[1]; e->st.filter_reject += back[2]; e->st.filter_nomatch += back[3];
+            // every submitted packet bumps exactly one of the three counters: what the filter skipped = submitted - kept
+            const uint64_t filtered_out = e->filter.n_rules ? back[1] + back[2] + back[3] - (uint64_t)m : 0;
+            size_t off = 0;
+            const int rc = ingest_device(e, e->d_expanded, m, &off);       // a chunk may be folded in several windows ("full" cuts)
+            if (rc == FA_FULL && off < m) {
+                // the cut is reported in snapshots: everything before the first record that was not folded, discarded ones included
+                uint32_t first_left = 0;
+                CU(cudaMemcpyAsync(&first_left, e->d_snap_src.get() + off, 4, cudaMemcpyDeviceToHost, e->stream));
+                CU(cudaStreamSynchronize(e->stream));
+                // discarded snapshots before the cut: first_left - off
+                // (with a filter the discarded / filtered split of a partially consumed chunk is not known: both count as discarded)
+                e->st.snaps_ingested += first_left;
+                e->st.snaps_discarded += first_left - off;
+                *took = first_left;
+                return rc;
+            }
+            if (rc != FA_OK) return rc;
+            e->st.snaps_ingested += c;
+            e->st.snaps_discarded += c - m - filtered_out;                  // fill_ethhdr's DISCARDs; the filter's skips are in its counters
+            *took = c;
+            return FA_OK;
+        });
 }
 
 int fa_set_flow_filter(fa_engine* e, const fa_filter_rule* rules, size_t n_rules, const fa_filter_cidr* peers, size_t n_peers) {
@@ -827,37 +846,24 @@ static int ingest_feature(fa_engine* e, int kind, const void* recs, size_t n, co
     if (!recs) return fail(FA_E_INVAL, "%s: null records", who);
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
+    if (int rc = check_headroom(e, n, who, "samples")) return rc;
     const size_t rec_bytes = kind == 1 ? fa::kDnsRecBytes : fa::kAddRecBytes;      // additional and packet-drop samples: 72 B
-    const PtrKind k = classify(recs);
-    if (k == PTR_DEVICE && (reinterpret_cast<uintptr_t>(recs) & 7)) return fail(FA_E_INVAL, "%s: device records must be 8-byte aligned", who);
-    // feature samples may create flows: never let the table pass 7/8 of its slots
-    int rc = sync_counters(e);
-    if (rc) return rc;
-    if (e->live_known + n > e->slots - e->slots / 8)
-        return fail(FA_E_2BIG, "%s: %zu samples could overfill the flow table (%llu live of %llu slots): evict first", who, n,
-                    (unsigned long long)e->live_known, (unsigned long long)e->slots);
-    if (k != PTR_DEVICE) { if (int arc = stage_alloc(e, k == PTR_PAGEABLE)) return arc; }
-    size_t done = 0;
-    while (done < n) {
-        const uint32_t c = (uint32_t)std::min<size_t>(n - done, k == PTR_DEVICE ? e->max_batch : stage_records(e));
-        const uint8_t* src = static_cast<const uint8_t*>(recs) + done * rec_bytes;
-        const uint8_t* d = src;
-        int sidx = -1;
-        if (k != PTR_DEVICE) {
-            if (int src_rc = stage_copy(e, src, (size_t)c * rec_bytes, k == PTR_PINNED, &sidx)) return src_rc;
-            d = e->d_stage[sidx];
-        }
-        e->st.kernel_launches += fa::launch_feature_fold(kind, d, c, e->table, ++e->epoch, e->feat_seq[kind], e->d_slot_of,
-                                                         e->d_ctr, e->sm_count, e->stream);
-        CU(cudaGetLastError());
-        e->feat_seq[kind] += c;
-        e->unsynced_records += c;
-        if (kind == 0) e->st.additional_ingested += c; else if (kind == 1) e->st.dns_ingested += c; else e->st.pkt_drops_ingested += c;
-        if (sidx >= 0) { if (int rel_rc = stage_release(e, sidx)) return rel_rc; }
-        done += c;
-    }
-    if (k != PTR_DEVICE) CU(cudaStreamSynchronize(e->copy_stream));   // the caller's buffer is not referenced after return
-    return FA_OK;
+    return ingest_caller_memory(
+        e, who, "records", 8, recs, n, rec_bytes, nullptr,
+        [&](size_t left, bool staged, size_t* c) {
+            *c = std::min<uint64_t>(left, staged ? stage_records(e) : e->max_batch);
+            return FA_OK;
+        },
+        [&](Chunk& ch, size_t c, size_t* took) {
+            e->st.kernel_launches += fa::launch_feature_fold(kind, ch.d, (uint32_t)c, e->table.view(), ++e->epoch, e->feat_seq[kind],
+                                                             e->d_slot_of, e->d_ctr, e->sm_count, e->stream);
+            CU(cudaGetLastError());
+            e->feat_seq[kind] += c;
+            e->unsynced_records += c;
+            if (kind == 0) e->st.additional_ingested += c; else if (kind == 1) e->st.dns_ingested += c; else e->st.pkt_drops_ingested += c;
+            *took = c;
+            return FA_OK;
+        });
 }
 
 int fa_ingest_additional(fa_engine* e, const void* recs, size_t n) { return ingest_feature(e, 0, recs, n, "fa_ingest_additional"); }
@@ -890,46 +896,31 @@ static int evict_swapped(fa_engine* e, const fa_evict_out* o, size_t cap, size_t
         if (live == 0) return FA_OK;
         if (!o->records) return fail(FA_E_INVAL, "fa_evict: null out_records");
         if (cap < live) return fail(FA_E_2BIG, "fa_evict: capacity %zu < %llu live flows", cap, (unsigned long long)live);
-        retired = e->table;
-        e->table = e->table_spare;                     // empty: the previous eviction deleted every flow in place
-        e->table_spare = retired;
+        retired = e->table.view();
+        std::swap(e->table, e->table_spare);           // the spare is empty: the previous eviction deleted every flow in place
         CU(cudaMemsetAsync(&e->d_ctr->live, 0, sizeof(unsigned long long), e->stream));
         CU(cudaEventRecord(e->ev_swap, e->stream));
         e->live_known = 0; e->unsynced_records = 0; e->ring_head = e->ring_tail;
         e->st.flows_evicted += live;
     }
     // from here on fa_ingest runs concurrently
-    const PtrKind k = classify(o->records);
-    uint8_t* d_out = static_cast<uint8_t*>(o->records);
-    if (k != PTR_DEVICE) {
-        if (e->evict_cap < live) {
-            cudaFree(e->d_evict); e->d_evict = nullptr; e->evict_cap = 0;
-            uint64_t want = std::max<uint64_t>(live, std::min<uint64_t>(e->cfg.max_entries, live * 2));
-            CU(cudaMalloc(&e->d_evict, want * fa::kRecBytes));
-            e->evict_cap = want;
-        }
-        d_out = e->d_evict;
-    }
+    uint8_t* d_out = nullptr;
+    if (int rc = evict_records_dst(e, o->records, live, &d_out)) return rc;
+    const bool staged = d_out != o->records;
     CU(cudaStreamWaitEvent(e->evict_stream, e->ev_swap, 0));
     CU(cudaMemsetAsync(&e->d_ctr_ev->evict_out, 0, sizeof(unsigned long long), e->evict_stream));
     const int launched = fa::launch_evict(retired, reinterpret_cast<uint4*>(d_out), nullptr, live, e->d_ctr_ev, e->sm_count, e->evict_stream);
     CU(cudaGetLastError());
-    if (k != PTR_DEVICE) CU(cudaMemcpyAsync(o->records, d_out, live * fa::kRecBytes, cudaMemcpyDeviceToHost, e->evict_stream));
+    if (staged) CU(cudaMemcpyAsync(o->records, d_out, live * fa::kRecBytes, cudaMemcpyDeviceToHost, e->evict_stream));
     CU(cudaMemcpyAsync(e->h_ev_out, &e->d_ctr_ev->evict_out, 8, cudaMemcpyDeviceToHost, e->evict_stream));
     CU(cudaStreamSynchronize(e->evict_stream));
     if (*e->h_ev_out != live)
         return fail(FA_E_CUDA, "fa_evict: table scan found %llu flows, counter says %llu", *e->h_ev_out, (unsigned long long)live);
-    if (k != PTR_DEVICE) {
-        if (o->present) memset(o->present, 0, live);
-        if (o->dns) memset(o->dns, 0, live * 64);
-        if (o->additional) memset(o->additional, 0, live * 32);
-        if (o->pkt_drops) memset(o->pkt_drops, 0, live * 32);
-        if (o->rtt_min) memset(o->rtt_min, 0, live * 8);
-    }
+    if (staged) zero_host_outputs(evict_outputs(e, o), live);   // double buffering is only available without feature tables
     {
         std::lock_guard<std::mutex> lk(e->mu);
         e->st.kernel_launches += launched;
-        if (k != PTR_DEVICE) e->st.d2h_bytes += live * fa::kRecBytes;
+        if (staged) e->st.d2h_bytes += live * fa::kRecBytes;
     }
     *n_out = (size_t)live;
     return FA_OK;
@@ -939,7 +930,6 @@ int fa_evict_ex(fa_engine* e, const fa_evict_out* o, size_t cap, size_t* n_out) 
     if (n_out) *n_out = 0;
     if (!e || !n_out || !o) return fail(FA_E_INVAL, "fa_evict: null argument");
     if (e->double_buffered) return evict_swapped(e, o, cap, n_out);
-    void* out_records = o->records; void* out_dns = o->dns; void* out_additional = o->additional; uint8_t* out_present = o->present;
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
     int rc = sync_counters(e);
@@ -947,77 +937,46 @@ int fa_evict_ex(fa_engine* e, const fa_evict_out* o, size_t cap, size_t* n_out) 
     const uint64_t live = e->live_known;
     e->st.evictions++;
     if (live == 0) return FA_OK;
-    if (!out_records) return fail(FA_E_INVAL, "fa_evict: null out_records");
+    if (!o->records) return fail(FA_E_INVAL, "fa_evict: null out_records");
     if (cap < live) return fail(FA_E_2BIG, "fa_evict: capacity %zu < %llu live flows", cap, (unsigned long long)live);
-    const bool feats = e->table.feat_add || e->table.feat_dns || e->table.feat_drop;
-    const PtrKind k = classify(out_records);
+    const bool feats = e->table.has_features();
     uint8_t* d_out = nullptr;
-    if (k == PTR_DEVICE) {
-        d_out = static_cast<uint8_t*>(out_records);
-    } else {
-        if (e->evict_cap < live) {
-            cudaFree(e->d_evict); e->d_evict = nullptr; e->evict_cap = 0;
-            uint64_t want = std::max<uint64_t>(live, std::min<uint64_t>(e->cfg.max_entries, live * 2));
-            CU(cudaMalloc(&e->d_evict, want * fa::kRecBytes));
-            e->evict_cap = want;
-        }
-        d_out = e->d_evict;
-    }
-    // feature outputs are staged on the device unless the caller handed device pointers
-    uint8_t *d_dns = nullptr, *d_add = nullptr, *d_drop = nullptr, *d_pres = nullptr;
-    unsigned long long* d_rmin = nullptr;
+    if ((rc = evict_records_dst(e, o->records, live, &d_out))) return rc;
+    const EvictOuts outs = evict_outputs(e, o);
+    std::array<uint8_t*, 5> d_feat{};                  // feature outputs are staged unless the caller handed device pointers
     if (feats) {
-        if (e->feat_evict_cap < live) {
-            cudaFree(e->d_evict_dns); cudaFree(e->d_evict_add); cudaFree(e->d_evict_present); cudaFree(e->d_slot_of_out);
-            cudaFree(e->d_evict_drop); cudaFree(e->d_evict_rttmin);
-            e->d_evict_dns = e->d_evict_add = e->d_evict_present = e->d_evict_drop = nullptr; e->d_evict_rttmin = nullptr;
-            e->d_slot_of_out = nullptr; e->feat_evict_cap = 0;
-            uint64_t want = std::max<uint64_t>(live, std::min<uint64_t>(e->cfg.max_entries, live * 2));
-            CU(cudaMalloc(&e->d_evict_dns, want * 64)); CU(cudaMalloc(&e->d_evict_add, want * 32));
-            CU(cudaMalloc(&e->d_evict_drop, want * 32)); CU(cudaMalloc(&e->d_evict_rttmin, want * 8));
-            CU(cudaMalloc(&e->d_evict_present, want)); CU(cudaMalloc(&e->d_slot_of_out, want * 4));
-            e->feat_evict_cap = want;
-        }
-        d_dns = out_dns ? (classify(out_dns) == PTR_DEVICE ? static_cast<uint8_t*>(out_dns) : e->d_evict_dns) : nullptr;
-        d_add = out_additional ? (classify(out_additional) == PTR_DEVICE ? static_cast<uint8_t*>(out_additional) : e->d_evict_add) : nullptr;
-        d_drop = o->pkt_drops ? (classify(o->pkt_drops) == PTR_DEVICE ? static_cast<uint8_t*>(o->pkt_drops) : e->d_evict_drop) : nullptr;
-        d_rmin = o->rtt_min ? (classify(o->rtt_min) == PTR_DEVICE ? reinterpret_cast<unsigned long long*>(o->rtt_min) : e->d_evict_rttmin) : nullptr;
-        d_pres = out_present ? (classify(out_present) == PTR_DEVICE ? out_present : e->d_evict_present) : nullptr;
+        for (const EvictOut& x : outs) { if ((rc = reserve_evict(e, *x.stage, live, x.width))) return rc; }
+        if ((rc = reserve_evict(e, e->d_slot_of_out, live, 4))) return rc;
+        for (size_t i = 0; i < outs.size(); i++)
+            if (outs[i].dst) d_feat[i] = classify(outs[i].dst) == PTR_DEVICE ? static_cast<uint8_t*>(outs[i].dst) : outs[i].stage->get();
     }
+    const fa::Table t = e->table.view();
+    uint32_t* slot_of_out = feats ? e->d_slot_of_out.get() : nullptr;
     CU(cudaMemsetAsync(&e->d_ctr->evict_out, 0, sizeof(unsigned long long), e->stream));
     if (e->cfg.mode == FA_MODE_KERNEL_MAP)
-        e->st.kernel_launches += fa::launch_kmap_evict(e->table, e->km_met, d_out, live, &e->d_ctr->evict_out,
-                                                       feats ? e->d_slot_of_out : nullptr, e->sm_count, e->stream);
+        e->st.kernel_launches += fa::launch_kmap_evict(t, e->km_met, d_out, live, &e->d_ctr->evict_out, slot_of_out, e->sm_count, e->stream);
     else
-        e->st.kernel_launches += fa::launch_evict(e->table, reinterpret_cast<uint4*>(d_out), feats ? e->d_slot_of_out : nullptr, live,
-                                                  e->d_ctr, e->sm_count, e->stream);
+        e->st.kernel_launches += fa::launch_evict(t, reinterpret_cast<uint4*>(d_out), slot_of_out, live, e->d_ctr, e->sm_count, e->stream);
     if (feats)
-        e->st.kernel_launches += fa::launch_evict_features(e->table, e->d_slot_of_out, live, d_out, d_dns, d_add, d_drop, d_rmin, d_pres,
+        e->st.kernel_launches += fa::launch_evict_features(t, slot_of_out, live, d_out, d_feat[0], d_feat[1], d_feat[2],
+                                                           reinterpret_cast<unsigned long long*>(d_feat[3]), d_feat[4],
                                                            e->sm_count, e->stream);
     CU(cudaGetLastError());
     CU(cudaMemsetAsync(&e->d_ctr->live, 0, sizeof(unsigned long long), e->stream));
-    if (k != PTR_DEVICE) {
-        CU(cudaMemcpyAsync(out_records, d_out, live * fa::kRecBytes, cudaMemcpyDeviceToHost, e->stream));
+    if (d_out != o->records) {
+        CU(cudaMemcpyAsync(o->records, d_out, live * fa::kRecBytes, cudaMemcpyDeviceToHost, e->stream));
         e->st.d2h_bytes += live * fa::kRecBytes;
     }
-    if (feats) {
-        if (out_dns && d_dns == e->d_evict_dns) { CU(cudaMemcpyAsync(out_dns, d_dns, live * 64, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += live * 64; }
-        if (out_additional && d_add == e->d_evict_add) { CU(cudaMemcpyAsync(out_additional, d_add, live * 32, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += live * 32; }
-        if (o->pkt_drops && d_drop == e->d_evict_drop) { CU(cudaMemcpyAsync(o->pkt_drops, d_drop, live * 32, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += live * 32; }
-        if (o->rtt_min && d_rmin == e->d_evict_rttmin) { CU(cudaMemcpyAsync(o->rtt_min, d_rmin, live * 8, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += live * 8; }
-        if (out_present && d_pres == e->d_evict_present) { CU(cudaMemcpyAsync(out_present, d_pres, live, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += live; }
+    for (size_t i = 0; i < outs.size(); i++) {
+        if (!d_feat[i] || d_feat[i] == outs[i].dst) continue;
+        CU(cudaMemcpyAsync(outs[i].dst, d_feat[i], live * outs[i].width, cudaMemcpyDeviceToHost, e->stream));
+        e->st.d2h_bytes += live * outs[i].width;
     }
     CU(cudaMemcpyAsync(e->h_ctr, e->d_ctr, sizeof(fa::Counters), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     if (e->h_ctr->evict_out != live)
         return fail(FA_E_CUDA, "fa_evict: table scan found %llu flows, counter says %llu", (unsigned long long)e->h_ctr->evict_out, (unsigned long long)live);
-    if (!feats) {
-        if (out_present && classify(out_present) != PTR_DEVICE) memset(out_present, 0, live);
-        if (out_dns && classify(out_dns) != PTR_DEVICE) memset(out_dns, 0, live * 64);
-        if (out_additional && classify(out_additional) != PTR_DEVICE) memset(out_additional, 0, live * 32);
-        if (o->pkt_drops && classify(o->pkt_drops) != PTR_DEVICE) memset(o->pkt_drops, 0, live * 32);
-        if (o->rtt_min && classify(o->rtt_min) != PTR_DEVICE) memset(o->rtt_min, 0, live * 8);
-    }
+    if (!feats) zero_host_outputs(outs, live);
     e->live_known = 0; e->unsynced_records = 0; e->ring_head = e->ring_tail;
     e->st.flows_evicted += live;
     *n_out = (size_t)live;
@@ -1035,12 +994,12 @@ int fa_drain_active(fa_engine* e, void* out_records_dev, size_t cap, size_t* n_o
     if (n_out) *n_out = 0;
     if (!e || !n_out || !out_records_dev) return fail(FA_E_INVAL, "fa_drain_active: null argument");
     if (classify(out_records_dev) != PTR_DEVICE) return fail(FA_E_INVAL, "fa_drain_active: out_records must be device memory");
-    if (e->table.feat_add || e->table.feat_dns || e->table.feat_drop) return fail(FA_E_INVAL, "fa_drain_active: not available with feature folds enabled");
+    if (e->table.has_features()) return fail(FA_E_INVAL, "fa_drain_active: not available with feature folds enabled");
     if (e->cfg.mode != FA_MODE_ACCOUNTER) return fail(FA_E_INVAL, "fa_drain_active: ACCOUNTER mode only");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
     CU(cudaMemsetAsync(&e->d_ctr->evict_out, 0, sizeof(unsigned long long), e->stream));
-    e->st.kernel_launches += fa::launch_evict(e->table, static_cast<uint4*>(out_records_dev), nullptr, cap, e->d_ctr,
+    e->st.kernel_launches += fa::launch_evict(e->table.view(), static_cast<uint4*>(out_records_dev), nullptr, cap, e->d_ctr,
                                               e->sm_count, e->stream, /*drain=*/true);
     CU(cudaGetLastError());
     int rc = sync_counters(e);
@@ -1054,12 +1013,12 @@ int fa_drain_active(fa_engine* e, void* out_records_dev, size_t cap, size_t* n_o
 
 int fa_drain_active_counted(fa_engine* e, void* out_records_dev, size_t cap, uint64_t* n_dev_out) {
     if (!e || !out_records_dev || !n_dev_out) return fail(FA_E_INVAL, "fa_drain_active_counted: null argument");
-    if (e->table.feat_add || e->table.feat_dns || e->table.feat_drop) return fail(FA_E_INVAL, "fa_drain_active_counted: not available with feature folds enabled");
+    if (e->table.has_features()) return fail(FA_E_INVAL, "fa_drain_active_counted: not available with feature folds enabled");
     if (e->cfg.mode != FA_MODE_ACCOUNTER) return fail(FA_E_INVAL, "fa_drain_active_counted: ACCOUNTER mode only");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
     CU(cudaMemsetAsync(&e->d_ctr->evict_out, 0, sizeof(unsigned long long), e->stream));
-    e->st.kernel_launches += fa::launch_evict(e->table, static_cast<uint4*>(out_records_dev), nullptr, cap, e->d_ctr,
+    e->st.kernel_launches += fa::launch_evict(e->table.view(), static_cast<uint4*>(out_records_dev), nullptr, cap, e->d_ctr,
                                               e->sm_count, e->stream, /*drain=*/true);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(n_dev_out, &e->d_ctr->evict_out, 8, cudaMemcpyDeviceToDevice, e->stream));
@@ -1143,33 +1102,30 @@ static int dnsc_init(fa_engine* e) {
     e->dnsc_chunk = std::min<uint64_t>(e->max_batch, 1ull << 20);
     uint64_t max_entries = kDnsMaxEntries;
     if (const char* me = getenv("FA_DNS_MAX_ENTRIES")) max_entries = std::max<uint64_t>(1, strtoull(me, nullptr, 0));
-    uint64_t kDnsSlots = 64; while (kDnsSlots < 4 * max_entries) kDnsSlots <<= 1;
-    e->dnsc_slots = kDnsSlots;
-    fa::DnsEntry* tab = nullptr;
-    CU(cudaMalloc(&tab, kDnsSlots * sizeof(fa::DnsEntry)));
-    CU(cudaMemsetAsync(tab, 0, kDnsSlots * sizeof(fa::DnsEntry), e->stream));
-    CU(cudaMalloc(&e->dnsc.ctr, fa::DNSC_N * 8));
-    CU(cudaMemsetAsync(e->dnsc.ctr, 0, fa::DNSC_N * 8, e->stream));
-    CU(cudaHostAlloc(&e->h_dnsc_ctr, fa::DNSC_N * 8, cudaHostAllocDefault));
-    CU(cudaMalloc(&e->d_dnsc_state, e->dnsc_chunk * 4));
-    CU(cudaMalloc(&e->d_dnsc_samples, e->dnsc_chunk * fa::kDnsRecBytes));
-    CU(cudaMalloc(&e->d_dnsc_out, e->dnsc_chunk * fa::kDnsRecBytes));
-    CU(cudaMalloc(&e->d_dnsc_warps, (e->dnsc_chunk + 31) / 32 * 4));
-    e->dnsc.mask = kDnsSlots - 1; e->dnsc.max_entries = max_entries;
-    e->dnsc.tab = tab;
+    e->dnsc_slots = pow2_at_least(64, 4 * max_entries);
+    if (int rc = alloc_zeroed(e, e->dnsc_tab, e->dnsc_slots * sizeof(fa::DnsEntry))) return rc;
+    if (int rc = alloc_zeroed(e, e->dnsc_ctr, fa::DNSC_N * 8)) return rc;
+    CU(e->h_dnsc_ctr.reserve(fa::DNSC_N * 8));
+    CU(e->d_dnsc_state.reserve(e->dnsc_chunk * 4));
+    CU(e->d_dnsc_samples.reserve(e->dnsc_chunk * fa::kDnsRecBytes));
+    CU(e->d_dnsc_out.reserve(e->dnsc_chunk * fa::kDnsRecBytes));
+    CU(e->d_dnsc_warps.reserve((e->dnsc_chunk + 31) / 32 * 4));
+    e->dnsc.mask = e->dnsc_slots - 1; e->dnsc.max_entries = max_entries;
+    e->dnsc.ctr = e->dnsc_ctr;
+    e->dnsc.tab = e->dnsc_tab;
     return FA_OK;
 }
 
 // move the pending queries into an empty table: the entries of answered queries are dropped
 static int dnsc_rebuild(fa_engine* e) {
-    if (!e->dnsc_spare) CU(cudaMalloc(&e->dnsc_spare, e->dnsc_slots * sizeof(fa::DnsEntry)));
-    CU(cudaMemsetAsync(e->dnsc_spare, 0, e->dnsc_slots * sizeof(fa::DnsEntry), e->stream));
+    if (int rc = alloc_zeroed(e, e->dnsc_spare, e->dnsc_slots * sizeof(fa::DnsEntry))) return rc;
     CU(cudaMemsetAsync(&e->dnsc.ctr[fa::DNSC_CREATED], 0, 8, e->stream));
     fa::DnsCorr to = e->dnsc;
     to.tab = e->dnsc_spare;
     e->st.kernel_launches += fa::launch_dns_rebuild(e->dnsc, to, e->sm_count, e->stream);
     CU(cudaGetLastError());
-    std::swap(e->dnsc.tab, e->dnsc_spare);
+    e->dnsc_tab.swap(e->dnsc_spare);
+    e->dnsc.tab = e->dnsc_tab;
     if (int rc = dnsc_sync(e)) return rc;
     e->dnsc_used = e->h_dnsc_ctr[fa::DNSC_CREATED];
     return FA_OK;
@@ -1184,48 +1140,36 @@ int fa_ingest_dns_packets(fa_engine* e, const void* pkts, size_t n) {
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
     if (int rc = dnsc_init(e)) return rc;
-    const PtrKind k = classify(pkts);
-    if (k == PTR_DEVICE && (reinterpret_cast<uintptr_t>(pkts) & 7)) return fail(FA_E_INVAL, "%s: device packets must be 8-byte aligned", who);
-    int rc = sync_counters(e);
-    if (rc) return rc;
-    if (e->live_known + n > e->slots - e->slots / 8)          // every packet may add a sample for a new flow
-        return fail(FA_E_2BIG, "%s: %zu packets could overfill the flow table (%llu live of %llu slots): evict first", who, n,
-                    (unsigned long long)e->live_known, (unsigned long long)e->slots);
-    if (k != PTR_DEVICE) { if (int arc = stage_alloc(e, k == PTR_PAGEABLE)) return arc; }
-    size_t done = 0;
-    while (done < n) {
-        // a chunk never takes more than a quarter of the table: with at most max_entries = slots / 4 present keys after a
-        // rebuild the table stays at most half full, so a probe sequence cannot run out
-        const uint64_t cmax = std::min<uint64_t>(e->dnsc_chunk, e->dnsc_slots / 4);
-        const uint32_t c = (uint32_t)std::min<size_t>(n - done, k == PTR_DEVICE ? cmax : std::min<uint64_t>(cmax, stage_records(e)));
-        if (e->dnsc_used + c > e->dnsc_slots / 2) { if (int rrc = dnsc_rebuild(e)) return rrc; }
-        const uint8_t* src = static_cast<const uint8_t*>(pkts) + done * fa::kDnsRecBytes;
-        const uint8_t* d = src;
-        int sidx = -1;
-        if (k != PTR_DEVICE) {
-            if (int src_rc = stage_copy(e, src, (size_t)c * fa::kDnsRecBytes, k == PTR_PINNED, &sidx)) return src_rc;
-            d = e->d_stage[sidx];
-        }
-        e->st.kernel_launches += fa::launch_dns_correlate(d, c, e->dnsc, e->d_dnsc_state, e->d_dnsc_samples, e->d_dnsc_warps, e->d_dnsc_out,
-                                                          e->sm_count, e->stream);
-        CU(cudaGetLastError());
-        if (sidx >= 0) { if (int rel_rc = stage_release(e, sidx)) return rel_rc; }
-        if (int src2 = dnsc_sync(e)) return src2;             // how many samples the chunk produced (sizes the fold)
-        e->dnsc_used += c;
-        const uint32_t m = (uint32_t)e->h_dnsc_ctr[fa::DNSC_EMITTED];
-        if (m) {
-            e->st.kernel_launches += fa::launch_feature_fold(1, e->d_dnsc_out, m, e->table, ++e->epoch, e->feat_seq[1], e->d_slot_of,
-                                                             e->d_ctr, e->sm_count, e->stream);
+    if (int rc = check_headroom(e, n, who, "packets")) return rc;     // every packet may add a sample for a new flow
+    return ingest_caller_memory(
+        e, who, "packets", 8, pkts, n, fa::kDnsRecBytes, nullptr,
+        [&](size_t left, bool staged, size_t* c) {
+            // a chunk never takes more than a quarter of the table: with at most max_entries = slots / 4 present keys after
+            // a rebuild the table stays at most half full, so a probe sequence cannot run out
+            const uint64_t cmax = std::min<uint64_t>(e->dnsc_chunk, e->dnsc_slots / 4);
+            *c = std::min<uint64_t>(left, staged ? std::min<uint64_t>(cmax, stage_records(e)) : cmax);
+            return e->dnsc_used + *c > e->dnsc_slots / 2 ? dnsc_rebuild(e) : FA_OK;
+        },
+        [&](Chunk& ch, size_t c, size_t* took) {
+            e->st.kernel_launches += fa::launch_dns_correlate(ch.d, (uint32_t)c, e->dnsc, e->d_dnsc_state, e->d_dnsc_samples,
+                                                              e->d_dnsc_warps, e->d_dnsc_out, e->sm_count, e->stream);
             CU(cudaGetLastError());
-            e->feat_seq[1] += m;
-            e->unsynced_records += m;
-            e->st.dns_ingested += m;
-        }
-        e->st.dns_packets_ingested += c;
-        done += c;
-    }
-    if (k != PTR_DEVICE) CU(cudaStreamSynchronize(e->copy_stream));
-    return FA_OK;
+            if (int rc = ch.release()) return rc;
+            if (int rc = dnsc_sync(e)) return rc;                     // how many samples the chunk produced (sizes the fold)
+            e->dnsc_used += c;
+            const uint32_t m = (uint32_t)e->h_dnsc_ctr[fa::DNSC_EMITTED];
+            if (m) {
+                e->st.kernel_launches += fa::launch_feature_fold(1, e->d_dnsc_out, m, e->table.view(), ++e->epoch, e->feat_seq[1],
+                                                                 e->d_slot_of, e->d_ctr, e->sm_count, e->stream);
+                CU(cudaGetLastError());
+                e->feat_seq[1] += m;
+                e->unsynced_records += m;
+                e->st.dns_ingested += m;
+            }
+            e->st.dns_packets_ingested += c;
+            *took = c;
+            return FA_OK;
+        });
 }
 
 int fa_purge_stale_dns(fa_engine* e, uint64_t mono_now_ns, uint64_t timeout_ns) {
@@ -1244,13 +1188,12 @@ int fa_cms_query(fa_engine* e, const void* keys, size_t n, uint64_t* est) {
     if (n == 0) return FA_OK;
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    struct DevBuf { void* p = nullptr; ~DevBuf() { if (p) cudaFree(p); } } keys_buf, est_buf;   // freed on every return path
-    CU(cudaMalloc(&keys_buf.p, n * 40 + 16));
-    CU(cudaMalloc(&est_buf.p, n * 8));
-    uint8_t* d_keys = static_cast<uint8_t*>(keys_buf.p);
-    unsigned long long* d_est = static_cast<unsigned long long*>(est_buf.p);
+    DevBuf<uint8_t> d_keys;
+    DevBuf<unsigned long long> d_est;
+    CU(d_keys.reserve(n * 40 + 16));
+    CU(d_est.reserve(n * 8));
     CU(cudaMemcpyAsync(d_keys, keys, n * 40, cudaMemcpyDefault, e->stream));
-    e->st.kernel_launches += fa::launch_cms_query(e->sk, reinterpret_cast<const uint4*>(d_keys), (uint32_t)n, d_est, e->stream);
+    e->st.kernel_launches += fa::launch_cms_query(e->sk, reinterpret_cast<const uint4*>(d_keys.get()), (uint32_t)n, d_est, e->stream);
     CU(cudaMemcpyAsync(est, d_est, n * 8, cudaMemcpyDefault, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     return FA_OK;
@@ -1268,12 +1211,11 @@ int fa_sketch_export(fa_engine* e, uint64_t* cms_out, size_t cms_words, uint8_t*
     }
     if (hll_out) {
         if (hll_regs < regs) return fail(FA_E_2BIG, "fa_sketch_export: hll buffer too small");
-        uint8_t* d_regs = nullptr;
-        CU(cudaMalloc(&d_regs, regs));
+        DevBuf<uint8_t> d_regs;
+        CU(d_regs.reserve(regs));
         e->st.kernel_launches += fa::launch_hll_pack(e->sk, d_regs, e->stream);
         CU(cudaMemcpyAsync(hll_out, d_regs, regs, cudaMemcpyDeviceToHost, e->stream));
         CU(cudaStreamSynchronize(e->stream));
-        cudaFree(d_regs);
     }
     CU(cudaStreamSynchronize(e->stream));
     return FA_OK;
@@ -1363,33 +1305,23 @@ int fa_pb_encode(fa_engine* e, const void* records, const void* dns, const void*
     if (p->n_ifaces && !p->ifaces) return fail(FA_E_INVAL, "fa_pb_encode: n_ifaces without ifaces");
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    struct DevBuf { void* p = nullptr; ~DevBuf() { if (p) cudaFree(p); } };
     // inputs: device pointers are used in place, host buffers are staged
-    DevBuf in_bufs[5], out_buf, keys_buf;
+    DevBuf<uint8_t> in_bufs[5], out_buf, keys_buf;
     const void* src[5] = {records, dns, additional, present, pkt_drops};
     const size_t width[5] = {fa::kRecBytes, 64, 32, 1, 32};
     const uint8_t* d_in[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     for (int i = 0; i < 5; i++) {
         if (!src[i]) continue;
         if (classify(src[i]) == PTR_DEVICE) { d_in[i] = static_cast<const uint8_t*>(src[i]); continue; }
-        CU(cudaMalloc(&in_bufs[i].p, n * width[i]));
-        CU(cudaMemcpyAsync(in_bufs[i].p, src[i], n * width[i], cudaMemcpyHostToDevice, e->stream));
+        CU(in_bufs[i].reserve(n * width[i]));
+        CU(cudaMemcpyAsync(in_bufs[i], src[i], n * width[i], cudaMemcpyHostToDevice, e->stream));
         e->st.h2d_bytes += n * width[i];
-        d_in[i] = static_cast<const uint8_t*>(in_bufs[i].p);
+        d_in[i] = in_bufs[i];
     }
-    if (e->pb_cap < n) {
-        cudaFree(e->d_pb_sizes); cudaFree(e->d_pb_offsets); cudaFree(e->d_pb_sums);
-        e->d_pb_sizes = nullptr; e->d_pb_offsets = nullptr; e->d_pb_sums = nullptr; e->pb_cap = 0;
-        CU(cudaMalloc(&e->d_pb_sizes, n * 4));
-        CU(cudaMalloc(&e->d_pb_offsets, (n + 1) * 8));
-        CU(cudaMalloc(&e->d_pb_sums, ((n + 1023) / 1024 + 1) * 8));
-        e->pb_cap = n;
-    }
-    if (p->n_ifaces > e->pb_ifaces_cap) {
-        cudaFree(e->d_pb_ifaces); e->d_pb_ifaces = nullptr; e->pb_ifaces_cap = 0;
-        CU(cudaMalloc(&e->d_pb_ifaces, (size_t)p->n_ifaces * sizeof(fa::PbIface)));
-        e->pb_ifaces_cap = p->n_ifaces;
-    }
+    CU(e->d_pb_sizes.reserve(n * 4));
+    CU(e->d_pb_offsets.reserve((n + 1) * 8));
+    CU(e->d_pb_sums.reserve(((n + 1023) / 1024 + 1) * 8));
+    CU(e->d_pb_ifaces.reserve((size_t)p->n_ifaces * sizeof(fa::PbIface)));
     if (p->n_ifaces) CU(cudaMemcpyAsync(e->d_pb_ifaces, p->ifaces, (size_t)p->n_ifaces * sizeof(fa::PbIface), cudaMemcpyHostToDevice, e->stream));
     fa::PbParams P{};
     P.now_unix_ns = p->now_unix_ns; P.mono_now_ns = p->mono_now_ns;
@@ -1408,10 +1340,10 @@ int fa_pb_encode(fa_engine* e, const void* records, const void* dns, const void*
     if (!out_bytes) return fail(FA_E_INVAL, "fa_pb_encode: null out_bytes");
     uint8_t* d_out = static_cast<uint8_t*>(out_bytes);
     const bool out_dev = classify(out_bytes) == PTR_DEVICE;
-    if (!out_dev) { CU(cudaMalloc(&out_buf.p, total ? total : 16)); d_out = static_cast<uint8_t*>(out_buf.p); }
+    if (!out_dev) { CU(out_buf.reserve(total ? total : 16)); d_out = out_buf; }
     uint8_t* d_keys = static_cast<uint8_t*>(keys_out);
     const bool keys_dev = keys_out && classify(keys_out) == PTR_DEVICE;
-    if (keys_out && !keys_dev) { CU(cudaMalloc(&keys_buf.p, n * 32)); d_keys = static_cast<uint8_t*>(keys_buf.p); }
+    if (keys_out && !keys_dev) { CU(keys_buf.reserve(n * 32)); d_keys = keys_buf; }
     e->st.kernel_launches += fa::launch_pb_write(in, (uint32_t)n, P, e->d_pb_offsets, e->d_pb_sizes, d_out, d_keys, e->stream);
     CU(cudaGetLastError());
     if (!out_dev) { CU(cudaMemcpyAsync(out_bytes, d_out, total, cudaMemcpyDeviceToHost, e->stream)); e->st.d2h_bytes += total; }
@@ -1442,11 +1374,8 @@ int fa_route(fa_engine* e, const void* recs, size_t n, uint32_t n_shards, void* 
     if (n > e->max_batch) return fail(FA_E_INVAL, "fa_route: n %zu > max_batch %llu", n, (unsigned long long)e->max_batch);
     std::lock_guard<std::mutex> lk(e->mu);
     CU(cudaSetDevice(e->device));
-    if (!e->d_route_tmp) {
-        const size_t ctas = (e->max_batch + 2047) / 2048;
-        CU(cudaMalloc(&e->d_route_tmp, (e->max_batch + 16 * ctas + 16) * 4));
-        CU(cudaMalloc(&e->d_route_counts, 16 * 8));
-    }
+    CU(e->d_route_tmp.reserve((e->max_batch + 16 * ((e->max_batch + 2047) / 2048) + 16) * 4));
+    CU(e->d_route_counts.reserve(16 * 8));
     e->st.kernel_launches += fa::launch_route(reinterpret_cast<const uint4*>(recs), (uint32_t)n, n_shards,
                                               reinterpret_cast<uint4*>(out), e->d_route_counts, e->d_route_tmp, e->sm_count, e->stream);
     CU(cudaGetLastError());

@@ -127,6 +127,69 @@ def test_random_streams_gpu():
     check_random(n_keys=5_000, n_base=80_000, n_feat=60_000, max_entries=1 << 17, max_batch=1 << 15)
 
 
+EVICT_OUT_BYTES = {"dns": 64, "additional": 32, "pkt_drops": 32, "rtt_min": 8, "present": 1}
+
+
+def evict_outputs(flags, where):
+    """Build one feature-laden state and evict it with each feature output placed as where[name]: "host", "device"
+    (fa_device_alloc: plain memory on the emulation) or None.  -> {name: bytes per flow, records sorted by key}."""
+    import ctypes as C
+    import netobserv_ebpf_agent_b200 as fa
+    from netobserv_ebpf_agent_b200._lib import EvictOut, check, lib
+    rng = np.random.default_rng(5)
+    base = gen_host(seed=41, n=500, n_keys=60, dist=1)
+    keys = np.concatenate([np.unique(base[:, :40], axis=0), keys_of(42, 8)])
+    with fa.FlowAggEngine(1 << 10, flags=flags, max_batch=512) as eng:
+        eng.ingest(base)
+        if flags:
+            eng.ingest_pkt_drops(make_drops(rng, keys, 300)); eng.ingest_additional(make_add(rng, keys, 300))
+            eng.ingest_dns(make_dns(rng, keys, 300))
+        n = eng.live_flows()
+        records, host, ptrs = np.zeros((n, 144), np.uint8), {}, {}
+        for name, width in EVICT_OUT_BYTES.items():
+            if where[name] == "host":
+                host[name] = np.full((n, width), 0xAB, np.uint8)             # stale bytes: must be overwritten
+                ptrs[name] = host[name].ctypes.data
+            elif where[name] == "device":
+                p = C.c_void_p()
+                check(lib().fa_device_alloc(eng._h, n * width, C.byref(p)))
+                ptrs[name] = p.value
+            else:
+                ptrs[name] = None
+        got = C.c_size_t(0)
+        check(lib().fa_evict_ex(eng._h, C.byref(EvictOut(records=records.ctypes.data, **ptrs)), n, C.byref(got)))
+        assert got.value == n
+        perm = O.sort_perm(records)
+        out = {"records": records[perm]}
+        for name, width in EVICT_OUT_BYTES.items():
+            if where[name] == "host":
+                out[name] = host[name][perm]
+            elif where[name] == "device":
+                out[name] = np.frombuffer(C.string_at(ptrs[name], n * width), np.uint8).reshape(n, width)[perm]
+                check(lib().fa_device_free(eng._h, ptrs[name]))
+    return out
+
+
+def test_evict_outputs_on_the_emulation(engine_emul):
+    """fa_evict_ex's five feature outputs stage through the device or are written in place: every mix of host, device
+    and absent outputs gives the same bytes, and without feature folds the host outputs come back zeroed."""
+    import netobserv_ebpf_agent_b200 as fa
+    flags = fa.FA_F_ENABLE_PKT_DROP | fa.FA_F_ENABLE_RTT | fa.FA_F_ENABLE_DNS
+    names = list(EVICT_OUT_BYTES)
+    want = evict_outputs(flags, dict.fromkeys(names, "host"))
+    assert want["present"].any() and want["rtt_min"].any()
+    mixes = [dict.fromkeys(names, "device"), dict.fromkeys(names, None),
+             dict(zip(names, ["host", "device", None, "device", "host"])), dict(zip(names, ["device", None, "host", "host", "device"]))]
+    for where in mixes:
+        got = evict_outputs(flags, where)
+        assert sorted(got) == sorted(["records"] + [k for k in names if where[k]])
+        for name, a in got.items():
+            assert np.array_equal(a, want[name]), (where, name)
+    plain = evict_outputs(0, dict.fromkeys(names, "host"))
+    assert all(not plain[name].any() for name in names)
+    assert len(plain["records"]) < len(want["records"])          # the feature samples created flows of their own
+
+
 def test_hot_keys_and_crowded_tiles_on_the_emulation(engine_emul):
     """K6 folds a tile's samples of one flow in shared memory before touching the table: a handful of keys (every tile is
     almost all duplicates) and a key set larger than the tile's election set both have to stay exact."""
